@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W              # our CUDA path (one rank per GPU)
     python bench.py --impl reference --steps K --warmup W      # the oracle port on host cores
+    python bench.py --steps K --warmup W --dump-outputs DIR    # + what the last timed step computed, as DIR/*.npy
 
 One *gradient step* of one agent = PER sample(B, beta) + n-step gather + RainbowDQN.learn
 (3 forwards, C51 projection, backward, clip, Adam, Polyak, noise reset) + update_priorities
@@ -210,9 +211,10 @@ def fused_population_step(agents, mem, nmem, support=None):
     """One learn step of every local agent against the shared HBM replay (agilerl_b200.training.
     population_learn).  The tree is read and written in agent order on one high-priority stream (the
     reference's sequential semantics); each agent's backward + optimiser runs on its own stream under
-    the next agents' forwards.  Tails are joined once, at the end of the timed region."""
+    the next agents' forwards.  Tails are joined once, at the end of the timed region.  Returns every
+    local agent's loss (device tensors)."""
     from agilerl_b200.training.population import population_learn
-    return population_learn(agents, mem, nmem, overlap=OVERLAP, join=False)[-1]
+    return population_learn(agents, mem, nmem, overlap=OVERLAP, join=False)
 
 
 def api_population_step(agents, mem, nmem, support, host_tr):
@@ -237,6 +239,24 @@ def api_population_step(agents, mem, nmem, support, host_tr):
 
 
 REPEATS = int(os.environ.get("B2RL_BENCH_REPEATS", "5"))
+DUMP_BYTES = 48 << 20                         # --dump-outputs budget over the whole population (limit: 64 MB)
+
+
+def dump_outputs(out_dir, agents, losses):
+    """What the last timed step handed back and left behind, per agent: its loss and its online and target
+    parameters after the step (float32; a fixed, seeded sample of the parameters where the population's
+    would exceed DUMP_BYTES).  Two builds run with the same arguments see the same inputs, so their dumps
+    compare array for array."""
+    os.makedirs(out_dir, exist_ok=True)
+    max_elems = DUMP_BYTES // (2 * POP * 4)
+    for agent, loss in zip(agents, losses):
+        arrays = {"loss": loss.detach().reshape(-1), "actor_params": agent.actor.buffers.params.detach(),
+                  "target_params": agent.actor_target.buffers.params.detach()}
+        for name, t in arrays.items():
+            a = t.float().cpu().numpy().reshape(-1)
+            if a.size > max_elems:
+                a = a[np.sort(np.random.default_rng(0).choice(a.size, max_elems, replace=False))]
+            np.save(os.path.join(out_dir, f"agent{agent.index}_{name}.npy"), a)
 
 
 def time_region(fn, steps, dist_on, finish=None, repeats=None):
@@ -787,7 +807,12 @@ def main():
     ap.add_argument("--workload", default="rainbow", choices=["rainbow", "ppo", "td3", "maddpg"],
                     help="rainbow: BASELINE configs[1] (the metric line the driver reads); td3: configs[2]; ppo: configs[3] "
                          "post-processing")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (each agent's loss and updated online "
+                         "and target parameters) as DIR/agent<i>_<name>.npy; rainbow workload, --impl ours")
     args = ap.parse_args()
+    if args.dump_outputs and (args.workload != "rainbow" or args.impl != "ours"):
+        ap.error("--dump-outputs is implemented for the rainbow workload with --impl ours")
     if args.workload == "ppo":
         return ppo_workload(args)
     if args.workload == "td3":
@@ -834,7 +859,11 @@ def main():
     support = torch.linspace(V_MIN, V_MAX, N_ATOMS).to(device)
 
     # ---- value: fused device path ------------------------------------------------------------
-    step_fn = lambda: fused_population_step(engines, mem, nmem, support)
+    last = {}
+
+    def step_fn():
+        last["losses"] = fused_population_step(engines, mem, nmem, support)
+
     for _ in range(max(args.warmup, 3)):
         step_fn()
     for a in engines:
@@ -854,6 +883,8 @@ def main():
     launches = (lib.b2rl_launch_count() - l0) // len(ms_all)
     clocks = sampler.stop() if rank == 0 else None
     value = POP * args.steps / (ms / 1e3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, engines, last["losses"])
 
     # ---- e2e: public API with host buffers ----------------------------------------------------
     e2e = None

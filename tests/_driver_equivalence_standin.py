@@ -2,18 +2,24 @@
 package's restatement of it (``agilerl_b200/training/train_off_policy.py`` — the driver the GPU box runs, where the reference
 does not exist) train the same seeded population on the same environment with the same stand-in kernels.  Stand-in outputs
 are deterministic functions of their inputs, so a faithful restatement yields IDENTICAL fitnesses, step counts, mutations,
-indices, call counts, exploration schedules and replay contents."""
+indices, call counts, exploration schedules and replay contents.
+
+The reference's run is stored in tests/golden/driver_equivalence.json; by default only our driver runs and is compared with
+it.  ``--record`` (tests/golden/make_golden.py, where the reference exists) runs both drivers, checks them against each other
+and prints the reference's run."""
 import json
+import math
 import os
 import random
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 MODE = sys.argv[1] if len(sys.argv) > 1 else "DQN"
+RECORD = "--record" in sys.argv
 helper = {"RAINBOW": "_reference_driver_rainbow_standin.py", "MADDPG": "_reference_ma_driver_standin.py"}.get(MODE, "_reference_driver_standin.py")
 src = open(os.path.join(ROOT, "tests", helper)).read()
 cut = {"RAINBOW": 'pop = create_population("Rainbow DQN"', "MADDPG": 'pop = create_population("MADDPG"'}.get(MODE, "import glob  # noqa: E402")
-sys.argv = [sys.argv[0], MODE]
+sys.argv = [sys.argv[0], MODE] + ([] if RECORD else ["--without-reference"])
 exec(compile(src[:src.index(cut)].replace("os.path.abspath(__file__)", repr(os.path.join(ROOT, "tests", helper))), helper, "exec"))
 from agilerl_b200.training import train_multi_agent_off_policy as ours_ma_driver  # noqa: E402
 from agilerl_b200.training import train_off_policy as ours_driver  # noqa: E402
@@ -56,9 +62,24 @@ def run(driver):
     return out
 
 
-if MODE == "MADDPG":
-    a, b = run(T.train_multi_agent_off_policy), run(ours_ma_driver)  # noqa: F821
+def same(x, y):
+    """Equal, floats to 1e-12 relative: the stored run comes from another process, maybe on another CPU, where a float sum over
+    a tensor may round its last bit differently."""
+    if isinstance(x, float) or isinstance(y, float):
+        return math.isclose(x, y, rel_tol=1e-12, abs_tol=1e-300)
+    if isinstance(x, dict):
+        return isinstance(y, dict) and x.keys() == y.keys() and all(same(x[k], y[k]) for k in x)
+    if isinstance(x, list):
+        return isinstance(y, list) and len(x) == len(y) and all(same(u, v) for u, v in zip(x, y))
+    return x == y
+
+
+if RECORD:
+    a = run(T.train_multi_agent_off_policy if MODE == "MADDPG" else T.train_off_policy)  # noqa: F821
+    print("REFERENCE " + json.dumps(a))
 else:
-    a, b = run(T.train_off_policy), run(ours_driver)                 # noqa: F821
-print("RESULT " + json.dumps({"equal": a == b, "diff": [k for k in a if a[k] != b[k]], "learn_calls": a["calls"].get("learn", a["calls"].get("loss")),
-                              "generations": len(a["fits"])}))
+    with open(os.path.join(ROOT, "tests", "golden", "driver_equivalence.json")) as f:
+        a = json.load(f)[MODE]
+b = json.loads(json.dumps(run(ours_ma_driver if MODE == "MADDPG" else ours_driver)))
+print("RESULT " + json.dumps({"equal": same(a, b), "diff": [k for k in a if not same(a[k], b.get(k))],
+                              "learn_calls": a["calls"].get("learn", a["calls"].get("loss")), "generations": len(a["fits"])}))

@@ -22,7 +22,9 @@ os.environ["B2RL_GRAPH"] = "0"                         # eager API path: graph c
 
 from oracle import refshim  # noqa: E402
 
-refshim.install()
+REFERENCE = "--without-reference" not in sys.argv     # tests/_driver_equivalence_standin.py: our driver alone
+if REFERENCE:
+    refshim.install()
 import agilerl_b200  # noqa: E402
 from agilerl_b200 import _lib  # noqa: E402
 from agilerl_b200.components import replay_buffer as rb  # noqa: E402
@@ -192,17 +194,18 @@ torch.cuda.Event = _Event
 rb._PinnedRing.sent = lambda self, k, dev: None
 
 agilerl_b200.install(include_driver=False)
-import inspect  # noqa: E402
-
-import agilerl.training.train_off_policy as T  # noqa: E402
-
-assert inspect.getsourcefile(T).startswith("/root/reference/"), inspect.getsourcefile(T)
 import agilerl_b200.algorithms as A  # noqa: E402
 import agilerl_b200.components as C  # noqa: E402
 import agilerl_b200.hpo as H  # noqa: E402
 
-assert T.RainbowDQN is A.RainbowDQN and T.PrioritizedReplayBuffer is C.PrioritizedReplayBuffer
-assert T.MultiStepReplayBuffer is C.MultiStepReplayBuffer and T.Sampler is C.Sampler
+if REFERENCE:
+    import inspect
+
+    import agilerl.training.train_off_policy as T
+
+    assert inspect.getsourcefile(T).startswith(refshim.REFERENCE_ROOT), inspect.getsourcefile(T)
+    assert T.RainbowDQN is A.RainbowDQN and T.PrioritizedReplayBuffer is C.PrioritizedReplayBuffer
+    assert T.MultiStepReplayBuffer is C.MultiStepReplayBuffer and T.Sampler is C.Sampler
 from agilerl_b200.compat import spaces  # noqa: E402
 from agilerl_b200.utils.utils import create_population  # noqa: E402
 

@@ -22,7 +22,9 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 from oracle import refshim  # noqa: E402
 
-refshim.install()
+REFERENCE = "--without-reference" not in sys.argv     # tests/_driver_equivalence_standin.py: our driver alone
+if REFERENCE:
+    refshim.install()
 import agilerl_b200  # noqa: E402
 from agilerl_b200 import _lib  # noqa: E402
 from agilerl_b200.components import replay_buffer as rb  # noqa: E402
@@ -103,16 +105,17 @@ torch.Tensor.pin_memory = lambda self: self
 rb._PinnedRing.sent = lambda self, k, dev: None
 
 agilerl_b200.install(include_driver=False)
-import inspect  # noqa: E402
-
-import agilerl.training.train_off_policy as T  # noqa: E402
-
-assert inspect.getsourcefile(T).startswith("/root/reference/"), inspect.getsourcefile(T)
 import agilerl_b200.algorithms as A  # noqa: E402
 import agilerl_b200.components as C  # noqa: E402
 import agilerl_b200.hpo as H  # noqa: E402
 
-assert T.DQN is A.DQN and T.TD3 is A.TD3 and T.ReplayBuffer is C.ReplayBuffer and T.Sampler is C.Sampler and T.Mutations is H.Mutations
+if REFERENCE:
+    import inspect
+
+    import agilerl.training.train_off_policy as T
+
+    assert inspect.getsourcefile(T).startswith(refshim.REFERENCE_ROOT), inspect.getsourcefile(T)
+    assert T.DQN is A.DQN and T.TD3 is A.TD3 and T.ReplayBuffer is C.ReplayBuffer and T.Sampler is C.Sampler and T.Mutations is H.Mutations
 from agilerl_b200.compat import spaces  # noqa: E402
 from agilerl_b200.utils.utils import create_population  # noqa: E402
 

@@ -19,7 +19,9 @@ os.environ["B2RL_MADDPG_GRAPH"] = "0"                  # eager learn call: graph
 
 from oracle import refshim  # noqa: E402
 
-refshim.install()
+REFERENCE = "--without-reference" not in sys.argv     # tests/_driver_equivalence_standin.py: our driver alone
+if REFERENCE:
+    refshim.install()
 import agilerl_b200  # noqa: E402
 from agilerl_b200 import _lib  # noqa: E402
 from agilerl_b200.components import replay_buffer as rb  # noqa: E402
@@ -65,17 +67,18 @@ torch.Tensor.pin_memory = lambda self: self
 rb._PinnedRing.sent = lambda self, k, dev: None
 
 agilerl_b200.install(include_driver=False)
-import inspect  # noqa: E402
-
-import agilerl.training.train_multi_agent_off_policy as T  # noqa: E402
-
-assert inspect.getsourcefile(T).startswith("/root/reference/"), inspect.getsourcefile(T)
 import agilerl_b200.algorithms as A  # noqa: E402
 import agilerl_b200.components as C  # noqa: E402
 import agilerl_b200.hpo as H  # noqa: E402
 
-assert T.MADDPG is A.MADDPG and T.MultiAgentReplayBuffer is C.MultiAgentReplayBuffer and T.Sampler is C.Sampler
-assert T.Mutations is H.Mutations and T.TournamentSelection is H.TournamentSelection
+if REFERENCE:
+    import inspect
+
+    import agilerl.training.train_multi_agent_off_policy as T
+
+    assert inspect.getsourcefile(T).startswith(refshim.REFERENCE_ROOT), inspect.getsourcefile(T)
+    assert T.MADDPG is A.MADDPG and T.MultiAgentReplayBuffer is C.MultiAgentReplayBuffer and T.Sampler is C.Sampler
+    assert T.Mutations is H.Mutations and T.TournamentSelection is H.TournamentSelection
 from agilerl_b200.compat import spaces  # noqa: E402
 from agilerl_b200.utils.utils import create_population  # noqa: E402
 

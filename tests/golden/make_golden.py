@@ -639,8 +639,75 @@ def gen_ma_replay():
     print("  multi-agent replay: oracle == reference on every sampled leaf (3 seeded batches, wrapped buffer)")
 
 
+def gen_api_surface():
+    """The reference's public signatures that tests/test_api_surface_cpu.py holds this package to: constructor parameters
+    (in order) of every replaced class, the defaults of the learners' constructors, the driver's parameters and the
+    multi-agent replay's method parameters."""
+    import inspect
+    import json
+
+    import agilerl.algorithms.maddpg as r_ma
+    import agilerl.components.multi_agent_replay_buffer as r_mb
+    import agilerl.hpo.mutation as r_mut
+    import agilerl.training.train_off_policy as r_train
+
+    def params(fn):
+        return [p for p in inspect.signature(fn).parameters if p != "self"]
+
+    def defaults(cls):
+        return {n: p.default for n, p in inspect.signature(cls.__init__).parameters.items()
+                if n not in ("self", "device") and p.default is not inspect.Parameter.empty}
+
+    classes = dict(ReplayBuffer=ReplayBuffer, MultiStepReplayBuffer=MultiStepReplayBuffer,
+                   PrioritizedReplayBuffer=PrioritizedReplayBuffer, RainbowDQN=RainbowDQN, DQN=DQN,
+                   TournamentSelection=TournamentSelection, Mutations=r_mut.Mutations, SumSegmentTree=SumSegmentTree,
+                   MinSegmentTree=MinSegmentTree, MADDPG=r_ma.MADDPG, MultiAgentReplayBuffer=r_mb.MultiAgentReplayBuffer)
+    out = {"ctor": {k: params(c.__init__) for k, c in classes.items()},
+           "defaults": {k: defaults(classes[k]) for k in ("RainbowDQN", "DQN", "MADDPG")},
+           "train_off_policy": params(r_train.train_off_policy),
+           "multi_agent_buffer_methods": {m: params(getattr(r_mb.MultiAgentReplayBuffer, m)) for m in
+                                          ("save_to_memory", "save_to_memory_single_env", "save_to_memory_vect_envs", "sample")}}
+    with open(os.path.join(HERE, "api_surface.json"), "w") as f:
+        json.dump(out, f, indent=1, sort_keys=True)
+    print("wrote api_surface.json")
+
+
+def gen_driver_equivalence():
+    """The reference's unchanged drivers on the seeded runs of tests/_driver_equivalence_standin.py (our restated driver is
+    checked against each run while recording)."""
+    import json
+    import subprocess
+
+    out = {}
+    for mode in ("DQN", "TD3", "RAINBOW", "MADDPG"):
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "_driver_equivalence_standin.py"), mode, "--record"],
+                           capture_output=True, text=True, check=True)
+        lines = dict(l.split(" ", 1) for l in p.stdout.splitlines() if l.startswith(("REFERENCE ", "RESULT ")))
+        assert json.loads(lines["RESULT"])["equal"], (mode, lines["RESULT"])
+        out[mode] = json.loads(lines["REFERENCE"])
+    with open(os.path.join(HERE, "driver_equivalence.json"), "w") as f:
+        json.dump(out, f, sort_keys=True)
+    print("wrote driver_equivalence.json: our restated drivers == the reference's")
+
+
+def gen_maddpg_host():
+    """The reference's ``MADDPG.test`` and ``get_action`` on the cases of tests/test_multi_agent_host_cpu.py."""
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import test_multi_agent_host_cpu as t
+    save("maddpg_host.npz", **t.reference_test_loop_outputs(), **t.reference_get_action_outputs())
+
+
 if __name__ == "__main__":
     torch.set_num_threads(1)   # deterministic CPU reductions while generating
+    if len(sys.argv) > 1 and sys.argv[1] == "api_surface":
+        gen_api_surface()
+        sys.exit(0)
+    if len(sys.argv) > 1 and sys.argv[1] == "drivers":
+        gen_driver_equivalence()
+        sys.exit(0)
+    if len(sys.argv) > 1 and sys.argv[1] == "maddpg_host":
+        gen_maddpg_host()
+        sys.exit(0)
     if len(sys.argv) > 1 and sys.argv[1] == "mutations":
         gen_mutations()
         sys.exit(0)
@@ -664,3 +731,6 @@ if __name__ == "__main__":
     gen_mutations()
     gen_maddpg()
     gen_ma_replay()
+    gen_api_surface()
+    gen_driver_equivalence()
+    gen_maddpg_host()

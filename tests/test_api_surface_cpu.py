@@ -1,27 +1,19 @@
-"""CPU, build container only: static drop-in check against the UNMODIFIED reference (imported
-through oracle.refshim): constructor parameters and public methods of every replaced class must be
-present with the same names (and order for constructors)."""
+"""CPU: static drop-in check against the UNMODIFIED reference (AgileRL 2.6.1): constructor parameters and public methods of
+every replaced class must be present with the same names (and order for constructors).  The reference's signatures are
+stored in tests/golden/api_surface.json (``python tests/golden/make_golden.py api_surface`` reads them from the reference)."""
 import inspect
+import json
+import os
 
 import pytest
 
-from oracle import refshim
-
-pytestmark = pytest.mark.skipif(not refshim.available(), reason="/root/reference not present (GPU box)")
+from conftest import GOLDEN
 
 
 @pytest.fixture(scope="module")
 def ref():
-    refshim.install()
-    import agilerl.algorithms.dqn as r_dqn
-    import agilerl.algorithms.dqn_rainbow as r_rb
-    import agilerl.components.replay_buffer as r_buf
-    import agilerl.components.sampler as r_samp
-    import agilerl.components.segment_tree as r_tree
-    import agilerl.hpo.mutation as r_mut
-    import agilerl.hpo.tournament as r_tour
-    import agilerl.training.train_off_policy as r_train
-    return dict(dqn=r_dqn, rb=r_rb, buf=r_buf, samp=r_samp, tree=r_tree, mut=r_mut, tour=r_tour, train=r_train)
+    with open(os.path.join(GOLDEN, "api_surface.json")) as f:
+        return json.load(f)
 
 
 def _ctor(cls):
@@ -36,16 +28,11 @@ def test_constructors_and_methods_match(ref):
     import agilerl_b200.algorithms as a
     import agilerl_b200.components as c
     import agilerl_b200.hpo as h
-    pairs = [
-        (ref["buf"].ReplayBuffer, c.ReplayBuffer), (ref["buf"].MultiStepReplayBuffer, c.MultiStepReplayBuffer),
-        (ref["buf"].PrioritizedReplayBuffer, c.PrioritizedReplayBuffer), (ref["rb"].RainbowDQN, a.RainbowDQN),
-        (ref["dqn"].DQN, a.DQN), (ref["tour"].TournamentSelection, h.TournamentSelection),
-        (ref["mut"].Mutations, h.Mutations), (ref["tree"].SumSegmentTree, c.SumSegmentTree),
-        (ref["tree"].MinSegmentTree, c.MinSegmentTree),
-    ]
-    for r, m in pairs:
-        rc, mc = _ctor(r), _ctor(m)
-        assert mc[:len(rc)] == rc or set(rc) <= set(mc), f"{r.__name__}: ctor {rc} vs {mc}"
+    ours = [c.ReplayBuffer, c.MultiStepReplayBuffer, c.PrioritizedReplayBuffer, a.RainbowDQN, a.DQN, h.TournamentSelection,
+            h.Mutations, c.SumSegmentTree, c.MinSegmentTree]
+    for m in ours:
+        rc, mc = ref["ctor"][m.__name__], _ctor(m)
+        assert mc[:len(rc)] == rc or set(rc) <= set(mc), f"{m.__name__}: ctor {rc} vs {mc}"
     need = {
         c.ReplayBuffer: {"add", "sample", "clear", "storage", "size", "is_full"},
         c.MultiStepReplayBuffer: {"add", "sample_from_indices"},
@@ -62,17 +49,15 @@ def test_constructors_and_methods_match(ref):
 
 def test_reference_defaults_match(ref):
     import agilerl_b200.algorithms as a
-    for r, m in ((ref["rb"].RainbowDQN, a.RainbowDQN), (ref["dqn"].DQN, a.DQN)):
-        rs, ms = inspect.signature(r.__init__).parameters, inspect.signature(m.__init__).parameters
-        for name, p in rs.items():
-            if name in ("self", "device") or p.default is inspect.Parameter.empty:
-                continue
-            assert ms[name].default == p.default, f"{r.__name__}.{name}: {ms[name].default} != {p.default}"
+    for m in (a.RainbowDQN, a.DQN):
+        ms = inspect.signature(m.__init__).parameters
+        for name, default in ref["defaults"][m.__name__].items():
+            assert ms[name].default == default, f"{m.__name__}.{name}: {ms[name].default} != {default}"
 
 
 def test_driver_signature_matches(ref):
     from agilerl_b200.training import train_off_policy as mine
-    rs = list(inspect.signature(ref["train"].train_off_policy).parameters)
+    rs = ref["train_off_policy"]
     ms = list(inspect.signature(mine).parameters)
     assert ms[:len(rs)] == rs, (rs, ms)
 
@@ -80,19 +65,14 @@ def test_driver_signature_matches(ref):
 def test_multi_agent_surface_matches(ref):
     """MADDPG / MultiAgentReplayBuffer (SURVEY 8f-4): same constructor parameters in the same order with the same
     defaults (``device`` aside), same public methods of the replay and the learner's hot-path methods."""
-    import agilerl.algorithms.maddpg as r_ma
-    import agilerl.components.multi_agent_replay_buffer as r_mb
     import agilerl_b200.algorithms as a
     import agilerl_b200.components as c
-    assert _ctor(a.MADDPG) == _ctor(r_ma.MADDPG)
-    assert _ctor(c.MultiAgentReplayBuffer) == _ctor(r_mb.MultiAgentReplayBuffer)
-    rs, ms = inspect.signature(r_ma.MADDPG.__init__).parameters, inspect.signature(a.MADDPG.__init__).parameters
-    for name, p in rs.items():
-        if name in ("self", "device") or p.default is inspect.Parameter.empty:
-            continue
-        assert ms[name].default == p.default, f"MADDPG.{name}: {ms[name].default} != {p.default}"
-    for name in ("save_to_memory", "save_to_memory_single_env", "save_to_memory_vect_envs", "sample"):
-        r_sig = list(inspect.signature(getattr(r_mb.MultiAgentReplayBuffer, name)).parameters)
-        m_sig = list(inspect.signature(getattr(c.MultiAgentReplayBuffer, name)).parameters)
+    assert _ctor(a.MADDPG) == ref["ctor"]["MADDPG"]
+    assert _ctor(c.MultiAgentReplayBuffer) == ref["ctor"]["MultiAgentReplayBuffer"]
+    ms = inspect.signature(a.MADDPG.__init__).parameters
+    for name, default in ref["defaults"]["MADDPG"].items():
+        assert ms[name].default == default, f"MADDPG.{name}: {ms[name].default} != {default}"
+    for name, r_sig in ref["multi_agent_buffer_methods"].items():
+        m_sig = [p for p in inspect.signature(getattr(c.MultiAgentReplayBuffer, name)).parameters if p != "self"]
         assert m_sig[:len(r_sig)] == r_sig, (name, r_sig, m_sig)
     assert {"learn", "get_action", "action_noise", "reset_action_noise", "soft_update", "test", "clone"} <= set(dir(a.MADDPG))

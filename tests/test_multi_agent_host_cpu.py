@@ -286,95 +286,168 @@ class _ParallelEnv:
         return {a: np.full(shape, self.t, np.float32) for a in self.ids}, rew, term, trunc, {a: {} for a in self.ids}
 
 
-@pytest.mark.parametrize("vect,sum_scores,max_steps", [(True, True, None), (True, False, 4), (False, True, None)])
-def test_maddpg_test_loop_matches_the_unmodified_reference(standin, vect, sum_scores, max_steps):
-    """``MADDPG.test`` (maddpg.py:756-875) against the reference's own method run through oracle/refshim on the same
-    environment with the same (stubbed) actions: identical fitness, NaN handling and episode bookkeeping."""
-    from oracle import refshim
-    if not refshim.available():
-        pytest.skip("/root/reference not present (GPU box)")
-    refshim.install()
-    import agilerl.algorithms.maddpg as r_ma
-    from agilerl_b200.algorithms import MADDPG
-    from agilerl_b200.compat import spaces
-    ids = ["agent_0", "agent_1", "agent_2"]
-    n = 3 if vect else None
+_TEST_LOOP_CASES = [(True, True, None), (True, False, 4), (False, True, None)]
+_TL_IDS = ["agent_0", "agent_1", "agent_2"]
 
+
+def _fake_get_action(n):
     def fake_get_action(self, obs, infos=None, **kw):
         rows = n or 1
-        act = {a: np.full((rows, 2), 0.1 * (k + 1), np.float32) for k, a in enumerate(ids)}
+        act = {a: np.full((rows, 2), 0.1 * (k + 1), np.float32) for k, a in enumerate(_TL_IDS)}
         return act, act
-    ours = MADDPG([spaces.Box(-1.0, 1.0, (4,), np.float32)] * 3, [spaces.Box(-1.0, 1.0, (2,), np.float32)] * 3, agent_ids=ids)
-    ours.get_action = fake_get_action.__get__(ours)
-    ref = r_ma.MADDPG.__new__(r_ma.MADDPG)                       # the method under test only needs these attributes
-    ref.agent_ids, ref.fitness = ids, []
-    ref.set_training_mode = lambda training: None
-    ref.get_action = fake_get_action.__get__(ref)
-    want = r_ma.MADDPG.test(ref, _ParallelEnv(ids, n), max_steps=max_steps, loop=2, sum_scores=sum_scores)
-    got = ours.test(_ParallelEnv(ids, n), max_steps=max_steps, loop=2, sum_scores=sum_scores)
-    np.testing.assert_array_equal(np.asarray(got), np.asarray(want))
-    np.testing.assert_array_equal(np.asarray(ours.fitness[-1]), np.asarray(ref.fitness[-1]))
+    return fake_get_action
+
+
+def reference_test_loop_outputs():
+    """``MADDPG.test`` of the unmodified reference (maddpg.py:756-875, run through oracle/refshim) on the cases of
+    test_maddpg_test_loop_matches_the_unmodified_reference; tests/golden/make_golden.py stores them in maddpg_host.npz."""
+    from oracle import refshim
+    refshim.install()
+    import agilerl.algorithms.maddpg as r_ma
+    out = {}
+    for vect, sum_scores, max_steps in _TEST_LOOP_CASES:
+        n = 3 if vect else None
+        ref = r_ma.MADDPG.__new__(r_ma.MADDPG)                   # the method under test only needs these attributes
+        ref.agent_ids, ref.fitness = _TL_IDS, []
+        ref.set_training_mode = lambda training: None
+        ref.get_action = _fake_get_action(n).__get__(ref)
+        key = f"test_loop/{vect}-{sum_scores}-{max_steps}"
+        out[key + "/scores"] = np.asarray(r_ma.MADDPG.test(ref, _ParallelEnv(_TL_IDS, n), max_steps=max_steps, loop=2,
+                                                         sum_scores=sum_scores))
+        out[key + "/fitness"] = np.asarray(ref.fitness[-1])
+    return out
+
+
+@pytest.mark.parametrize("vect,sum_scores,max_steps", _TEST_LOOP_CASES)
+def test_maddpg_test_loop_matches_the_unmodified_reference(standin, vect, sum_scores, max_steps):
+    """``MADDPG.test`` (maddpg.py:756-875) against the reference's own method (its results stored in maddpg_host.npz) on the
+    same environment with the same (stubbed) actions: identical fitness, NaN handling and episode bookkeeping."""
+    from agilerl_b200.algorithms import MADDPG
+    from agilerl_b200.compat import spaces
+    g = load_golden("maddpg_host.npz")
+    key = f"test_loop/{vect}-{sum_scores}-{max_steps}"
+    n = 3 if vect else None
+    ours = MADDPG([spaces.Box(-1.0, 1.0, (4,), np.float32)] * 3, [spaces.Box(-1.0, 1.0, (2,), np.float32)] * 3, agent_ids=_TL_IDS)
+    ours.get_action = _fake_get_action(n).__get__(ours)
+    got = ours.test(_ParallelEnv(_TL_IDS, n), max_steps=max_steps, loop=2, sum_scores=sum_scores)
+    np.testing.assert_array_equal(np.asarray(got), g[key + "/scores"])
+    np.testing.assert_array_equal(np.asarray(ours.fitness[-1]), g[key + "/fitness"])
     assert ours.training is False
+
+
+_GA_IDS = ["a", "b"]
+
+
+def _ga_spaces(sp):
+    return ([sp.Box(-1.0, 1.0, (6,), np.float32), sp.Box(-1.0, 1.0, (4,), np.float32)],
+            [sp.Box(-2.0, 3.0, (3,), np.float32), sp.Box(-0.5, 1.5, (3,), np.float32)])
+
+
+def _ga_calls():
+    """(training, obs, infos, seed) of every ``get_action`` call: three plain ones, then actions dictated by the environment
+    (maddpg.py:518-529): NaN rows are the agent's own, the rest overwrite."""
+    g = torch.Generator().manual_seed(0)
+    calls = []
+    for training in (True, True, False):
+        calls.append((training, {"a": torch.randn(4, 6, generator=g).numpy(), "b": torch.randn(4, 4, generator=g).numpy()},
+                      None, 77))
+    eda = np.full((4, 3), np.nan)
+    eda[1] = [0.5, -0.25, 1.0]
+    eda[3] = [-2.0, 3.0, 0.0]
+    infos = {"a": {"env_defined_actions": eda}, "b": {"env_defined_actions": np.full((4, 3), np.nan)}}
+    calls.append((False, {"a": torch.randn(4, 6, generator=g).numpy(), "b": torch.randn(4, 4, generator=g).numpy()}, infos, 78))
+    return calls
+
+
+def _copy_args(obs, infos):
+    return ({k: v.copy() for k, v in obs.items()},
+            None if infos is None else {k: {kk: vv.copy() for kk, vv in v.items()} for k, v in infos.items()})
+
+
+def reference_get_action_outputs():
+    """``get_action`` / ``action_noise`` / ``reset_action_noise`` of the unmodified reference (maddpg.py:428-558) on the calls
+    of ``_ga_calls``, with what its actors were handed and returned; tests/golden/make_golden.py stores them in
+    maddpg_host.npz."""
+    from oracle import refshim
+    refshim.install()
+    import agilerl.algorithms.maddpg as r_ma
+    from gymnasium import spaces as r_spaces
+    out = {}
+    for ou_noise in (True, False):
+        pre = f"get_action/{ou_noise}"
+        torch.manual_seed(5)
+        ref = r_ma.MADDPG(*_ga_spaces(r_spaces), agent_ids=_GA_IDS, O_U_noise=ou_noise, vect_noise_dim=4, expl_noise=0.3,
+                          device="cpu")
+        seen = {a: [] for a in _GA_IDS}
+        for a in _GA_IDS:
+            actor = ref.actors[a]
+            out[f"{pre}/{a}/action_low"], out[f"{pre}/{a}/action_high"] = actor.action_low.cpu().numpy(), actor.action_high.cpu().numpy()
+            out[f"{pre}/{a}/output_activation"] = np.asarray(actor.output_activation)
+        cls = type(ref.actors[_GA_IDS[0]])
+        call = cls.__call__                  # the actors override __call__, so module hooks do not see their calls
+
+        def recording_call(self, x, *args, **kw):
+            y = call(self, x, *args, **kw)
+            a = next(a for a in _GA_IDS if ref.actors[a] is self)
+            seen[a].append((x.detach().cpu().numpy().copy(), y.detach().cpu().numpy().copy()))
+            return y
+        cls.__call__ = recording_call
+        try:
+            for c, (training, obs, infos, seed) in enumerate(_ga_calls()):
+                ref.set_training_mode(training)
+                torch.manual_seed(seed)
+                want_p, want_r = ref.get_action(*_copy_args(obs, infos))
+                for a in _GA_IDS:
+                    out[f"{pre}/{c}/{a}/processed"], out[f"{pre}/{c}/{a}/raw"] = np.asarray(want_p[a]), np.asarray(want_r[a])
+        finally:
+            cls.__call__ = call
+        for a in _GA_IDS:
+            out[f"{pre}/{a}/actor_in"] = np.stack([x for x, _ in seen[a]])
+            out[f"{pre}/{a}/actor_out"] = np.stack([y for _, y in seen[a]])
+        ref.reset_action_noise([1, 3])
+        for a in _GA_IDS:
+            out[f"{pre}/{a}/noise_after_reset"] = ref.current_noise[a].cpu().numpy()
+    return out
 
 
 @pytest.mark.parametrize("ou_noise", [True, False])
 def test_maddpg_get_action_noise_and_rescaling_match_the_unmodified_reference(standin, ou_noise):
     """``get_action`` / ``action_noise`` (maddpg.py:428-558) around the actor forward: exploration noise from torch's global
     generator (Ornstein-Uhlenbeck state carried across calls, or Gaussian), clamp to [-1, 1], rescale to the action bounds (kept quirk: the LAST agent's bounds for every agent, maddpg.py:504-511) —
-    the real reference object next to ours, our actors stubbed to return the reference actors' outputs."""
-    from oracle import refshim
-    if not refshim.available():
-        pytest.skip("/root/reference not present (GPU box)")
-    refshim.install()
-    import agilerl.algorithms.maddpg as r_ma
-    from gymnasium import spaces as r_spaces
+    against the reference object's results (stored in maddpg_host.npz), our actors stubbed to return what the reference actors
+    returned on the same inputs."""
     from agilerl_b200.algorithms import MADDPG
     from agilerl_b200.compat import spaces
-    ids = ["a", "b"]
-    mk = lambda sp: ([sp.Box(-1.0, 1.0, (6,), np.float32), sp.Box(-1.0, 1.0, (4,), np.float32)],
-                     [sp.Box(-2.0, 3.0, (3,), np.float32), sp.Box(-0.5, 1.5, (3,), np.float32)])
+    g = load_golden("maddpg_host.npz")
+    pre = f"get_action/{ou_noise}"
     torch.manual_seed(5)
-    ref = r_ma.MADDPG(*mk(r_spaces), agent_ids=ids, O_U_noise=ou_noise, vect_noise_dim=4, expl_noise=0.3, device="cpu")
-    ours = MADDPG(*mk(spaces), agent_ids=ids, O_U_noise=ou_noise, vect_noise_dim=4, expl_noise=0.3)
+    ours = MADDPG(*_ga_spaces(spaces), agent_ids=_GA_IDS, O_U_noise=ou_noise, vect_noise_dim=4, expl_noise=0.3)
 
     class Stub:
-        def __init__(self, actor):
-            self.actor, self.action_low, self.action_high = actor, actor.action_low.cpu(), actor.action_high.cpu()
-            self.output_activation = actor.output_activation
+        def __init__(self, a):
+            self.a, self.calls = a, 0
+            self.action_low = torch.from_numpy(g[f"{pre}/{a}/action_low"])
+            self.action_high = torch.from_numpy(g[f"{pre}/{a}/action_high"])
+            self.output_activation = str(g[f"{pre}/{a}/output_activation"])
 
         def __call__(self, obs):
-            with torch.no_grad():
-                return self.actor(obs.cpu())
-    ours.actors = {a: Stub(ref.actors[a]) for a in ids}
-    g = torch.Generator().manual_seed(0)
-    for training in (True, True, False):
-        ref.set_training_mode(training); ours.set_training_mode(training)
-        obs = {"a": torch.randn(4, 6, generator=g).numpy(), "b": torch.randn(4, 4, generator=g).numpy()}
-        torch.manual_seed(77)
-        want_p, want_r = ref.get_action({k: v.copy() for k, v in obs.items()})
-        torch.manual_seed(77)
-        got_p, got_r = ours.get_action({k: v.copy() for k, v in obs.items()})
-        for a in ids:
-            np.testing.assert_array_equal(got_r[a], want_r[a], err_msg=f"raw {a} training={training}")
-            np.testing.assert_array_equal(got_p[a], want_p[a], err_msg=f"processed {a} training={training}")
-    # actions dictated by the environment (maddpg.py:518-529): NaN rows are the agent's own, the rest overwrite — and the
-    # overwritten dict also comes back as the "raw" actions (kept quirk)
-    eda = np.full((4, 3), np.nan)
-    eda[1] = [0.5, -0.25, 1.0]
-    eda[3] = [-2.0, 3.0, 0.0]
-    infos = {"a": {"env_defined_actions": eda}, "b": {"env_defined_actions": np.full((4, 3), np.nan)}}
-    obs = {"a": torch.randn(4, 6, generator=g).numpy(), "b": torch.randn(4, 4, generator=g).numpy()}
-    torch.manual_seed(78)
-    want_p, want_r = ref.get_action({k: v.copy() for k, v in obs.items()}, infos={k: {kk: vv.copy() for kk, vv in v.items()} for k, v in infos.items()})
-    torch.manual_seed(78)
-    got_p, got_r = ours.get_action({k: v.copy() for k, v in obs.items()}, infos={k: {kk: vv.copy() for kk, vv in v.items()} for k, v in infos.items()})
-    for a in ids:
-        np.testing.assert_array_equal(got_p[a], want_p[a], err_msg=f"env-defined processed {a}")
-        np.testing.assert_array_equal(got_r[a], want_r[a], err_msg=f"env-defined raw {a}")
+            k, self.calls = self.calls, self.calls + 1
+            np.testing.assert_array_equal(obs.cpu().numpy(), g[f"{pre}/{self.a}/actor_in"][k])
+            return torch.from_numpy(g[f"{pre}/{self.a}/actor_out"][k].copy())
+    ours.actors = {a: Stub(a) for a in _GA_IDS}
+    for c, (training, obs, infos, seed) in enumerate(_ga_calls()):
+        ours.set_training_mode(training)
+        torch.manual_seed(seed)
+        got_p, got_r = ours.get_action(*_copy_args(obs, infos))
+        for a in _GA_IDS:
+            np.testing.assert_array_equal(got_r[a], g[f"{pre}/{c}/{a}/raw"], err_msg=f"raw {a} call {c} training={training}")
+            np.testing.assert_array_equal(got_p[a], g[f"{pre}/{c}/{a}/processed"], err_msg=f"processed {a} call {c}")
+    # the environment's actions overwrite the processed ones, and the overwritten dict also comes back as the "raw" actions
     np.testing.assert_array_equal(got_p["a"][1], [0.5, -0.25, 1.0])
-    ref.reset_action_noise([1, 3]); ours.reset_action_noise([1, 3])
-    for a in ids:
-        assert torch.equal(ours.current_noise[a], ref.current_noise[a])
+    assert all(s.calls == len(g[f"{pre}/{a}/actor_in"]) for a, s in ours.actors.items())
+    ours.reset_action_noise([1, 3])
+    for a in _GA_IDS:
+        np.testing.assert_array_equal(ours.current_noise[a].cpu().numpy(), g[f"{pre}/{a}/noise_after_reset"])
 
 
 def test_rl_hyperparameter_and_parameter_mutations_on_a_maddpg_member(standin):
