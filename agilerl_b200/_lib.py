@@ -94,6 +94,7 @@ class MaddpgCfg(Structure):
         ("gamma", c_double), ("tau", c_double),
         ("lr_actor", c_double), ("lr_critic", c_double), ("beta1", c_double), ("beta2", c_double), ("adam_eps", c_double),
         ("bc1_actor", c_double), ("bc2_actor", c_double), ("bc1_critic", c_double), ("bc2_critic", c_double),
+        ("twin", c_int32), ("critic_only", c_int32),
     ]
 
 
@@ -105,6 +106,9 @@ class MaddpgBufs(Structure):
         ("critic_grads", c_void_p * B2RL_MAX_AGENTS), ("critic_m", c_void_p * B2RL_MAX_AGENTS), ("critic_v", c_void_p * B2RL_MAX_AGENTS),
         ("obs", c_void_p), ("next_obs", c_void_p), ("action", c_void_p), ("reward", c_void_p), ("done", c_void_p),
         ("losses", c_void_p), ("workspace", c_void_p), ("workspace_bytes", c_size_t), ("step_state", c_void_p),
+        ("critic2", c_void_p * B2RL_MAX_AGENTS), ("critic2_target", c_void_p * B2RL_MAX_AGENTS),
+        ("critic2_grads", c_void_p * B2RL_MAX_AGENTS), ("critic2_m", c_void_p * B2RL_MAX_AGENTS),
+        ("critic2_v", c_void_p * B2RL_MAX_AGENTS), ("actor_step_state", c_void_p),
     ]
 
 
@@ -148,11 +152,13 @@ _SIGS = {
     "b2rl_graph_begin": ([c_void_p], c_int),
     "b2rl_graph_end": ([c_void_p, POINTER(c_void_p)], c_int),
     "b2rl_graph_launch": ([c_void_p, POINTER(StepState), c_void_p], c_int),
+    "b2rl_graph_launch_states": ([c_void_p, c_void_p, c_void_p, c_int, c_void_p], c_int),
     "b2rl_graph_kernel_count": ([c_void_p, POINTER(c_int)], c_int),
     "b2rl_graph_destroy": ([c_void_p], c_int),
     "b2rl_ddpg_workspace_bytes": ([POINTER(NetDesc), POINTER(NetDesc), c_int64, POINTER(c_size_t)], c_int),
     "b2rl_ddpg_learn": ([POINTER(NetDesc), POINTER(NetDesc), POINTER(DdpgCfg), POINTER(DdpgBufs), c_void_p], c_int),
     "b2rl_maddpg_workspace_bytes": ([c_void_p, c_void_p, c_int, c_int64, POINTER(c_size_t)], c_int),
+    "b2rl_maddpg_workspace_bytes_cfg": ([c_void_p, c_void_p, POINTER(MaddpgCfg), POINTER(c_size_t)], c_int),
     "b2rl_maddpg_learn": ([c_void_p, c_void_p, POINTER(MaddpgCfg), POINTER(MaddpgBufs), c_void_p], c_int),
     "b2rl_gaussian_mutate": ([c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_uint64, c_uint64,
                               c_double, c_int64, c_void_p], c_int),

@@ -42,7 +42,11 @@ class _LearnPlan:
     """Static batch buffers + the captured graph of one ``b2rl_maddpg_learn`` call for a batch size: ~130 dependent
     launches (four concurrent per-agent chains) replayed as ONE graph launch.  What changes between steps — Adam's bias
     corrections — lives in a ``b2rl_step_state`` on the device, rewritten by the graph's first node from the host's
-    double arithmetic, so a replay is bit-identical to the eager call (tests/test_maddpg_gpu.py)."""
+    double arithmetic, so a replay is bit-identical to the eager call (tests/test_maddpg_gpu.py).
+
+    ``graphs`` holds one graph per step kind (``critic_only``): MADDPG only ever has the full step (``graph``); MATD3 also
+    captures its critic-only call, and its full step writes a second state block for the actors (``actor_state_*``), whose
+    optimisers have stepped fewer times than the critics'."""
 
     def __init__(self, agent, B: int):
         dev, n = agent._dev, agent.n_agents
@@ -53,17 +57,24 @@ class _LearnPlan:
         self.state_host = _lib.StepState()
         self.state_ref = ctypes.byref(self.state_host)
         self.state_dev = torch.zeros(ctypes.sizeof(_lib.StepState), dtype=torch.uint8, device=dev)
-        self.graph = None
+        self.actor_state_host = _lib.StepState()
+        self.actor_state_dev = torch.zeros(ctypes.sizeof(_lib.StepState), dtype=torch.uint8, device=dev)
+        self.graphs: dict = {}
         self._fields = [self.obs, self.action, self.reward, self.next_obs, self.done]
 
     def fields(self):
         """The static buffers in the replay's field order (obs, action, reward, next_obs, done)."""
         return self._fields
 
+    @property
+    def graph(self):
+        """The captured full step (actor and critic updates, soft updates)."""
+        return self.graphs.get(False)
+
     def destroy(self) -> None:
-        if self.graph:
-            _lib.load().b2rl_graph_destroy(self.graph)
-            self.graph = None
+        for g in self.graphs.values():
+            _lib.load().b2rl_graph_destroy(g)
+        self.graphs = {}
 
 
 class _AgentOptimizers(OrderedDict):
@@ -83,6 +94,9 @@ def concatenate_spaces(space_list) -> spaces.Box:
 
 
 class MADDPG(EvolvableAlgorithm):
+    # (networks, targets, optimisers) of each centralised critic set; MATD3 has two
+    _CRITIC_SETS = (("critics", "critic_targets", "critic_optimizers"),)
+
     def __init__(self, observation_spaces, action_spaces, agent_ids: list[str] | None = None, O_U_noise: bool = True,
                  expl_noise: float = 0.1, vect_noise_dim: int = 1, mean_noise: float = 0.0, theta: float = 0.15,
                  dt: float = 1e-2, index: int = 0, hp_config: HyperparameterConfig | None = None,
@@ -90,7 +104,7 @@ class MADDPG(EvolvableAlgorithm):
                  lr_critic: float = 0.01, learn_step: int = 5, gamma: float = 0.95, tau: float = 0.01, mut: str | None = None,
                  normalize_images: bool = True, actor_networks=None, critic_networks=None, device: str = "cuda",
                  accelerator: Any | None = None, torch_compiler: str | None = None, wrap: bool = True) -> None:
-        super().__init__(index, hp_config, device, accelerator, torch_compiler, name="MADDPG")
+        super().__init__(index, hp_config, device, accelerator, torch_compiler, name=type(self).__name__)
         if isinstance(observation_spaces, (spaces.Dict, dict)):
             agent_ids = list(observation_spaces.keys()) if agent_ids is None else agent_ids
             observation_spaces = [observation_spaces[a] for a in agent_ids]
@@ -156,32 +170,39 @@ class MADDPG(EvolvableAlgorithm):
         mk_c = lambda: MultiInputContinuousQNetwork(self.observation_space, all_act, latent_dim=latent_dim,
                                                     head_config=critic_head, device=self.device)
         self.actors = OrderedDict((a, mk_a(a)) for a in self.agent_ids)
-        self.critics = OrderedDict((a, mk_c()) for a in self.agent_ids)
+        for net, _, _ in self._CRITIC_SETS:
+            setattr(self, net, OrderedDict((a, mk_c()) for a in self.agent_ids))
         self.actor_targets = OrderedDict((a, mk_a(a)) for a in self.agent_ids)
-        self.critic_targets = OrderedDict((a, mk_c()) for a in self.agent_ids)
+        for _, tgt, _ in self._CRITIC_SETS:
+            setattr(self, tgt, OrderedDict((a, mk_c()) for a in self.agent_ids))
         for a in self.agent_ids:
             self.actors[a].encoder.disable_mutations()                                   # maddpg.py:324-326
             self.actor_targets[a].load_state_dict(self.actors[a].state_dict())
-            self.critic_targets[a].load_state_dict(self.critics[a].state_dict())
+            for net, tgt, _ in self._CRITIC_SETS:
+                getattr(self, tgt)[a].load_state_dict(getattr(self, net)[a].state_dict())
         self.register_network_group(NetworkGroup(eval_network="actors", shared_networks="actor_targets", policy=True))
-        self.register_network_group(NetworkGroup(eval_network="critics", shared_networks="critic_targets"))
+        for net, tgt, _ in self._CRITIC_SETS:
+            self.register_network_group(NetworkGroup(eval_network=net, shared_networks=tgt))
         self.registry.register_optimizer(OptimizerConfig(name="actor_optimizers", networks=["actors"], lr="lr_actor"))
-        self.registry.register_optimizer(OptimizerConfig(name="critic_optimizers", networks=["critics"], lr="lr_critic"))
+        for net, _, opt in self._CRITIC_SETS:
+            self.registry.register_optimizer(OptimizerConfig(name=opt, networks=[net], lr="lr_critic"))
         self._bind_engine()
 
     # -- engine state ------------------------------------------------------------------------------------
     def _bind_engine(self, keep: dict | None = None) -> None:
         self.actor_optimizers = _AgentOptimizers((a, _AdamState(self.actors[a], self.lr_actor)) for a in self.agent_ids)
-        self.critic_optimizers = _AgentOptimizers((a, _AdamState(self.critics[a], self.lr_critic)) for a in self.agent_ids)
+        for net, _, opt in self._CRITIC_SETS:
+            setattr(self, opt, _AgentOptimizers((a, _AdamState(getattr(self, net)[a], self.lr_critic)) for a in self.agent_ids))
         if keep:
-            for a in self.agent_ids:
-                self.actor_optimizers[a].load_state_dict(keep["actors"][a])
-                self.critic_optimizers[a].load_state_dict(keep["critics"][a])
+            for name in self._opt_names():
+                for a in self.agent_ids:
+                    getattr(self, name)[a].load_state_dict(keep[name][a])
         n = self.n_agents
+        critics = getattr(self, self._CRITIC_SETS[0][0])        # every critic set shares one architecture (one layer table)
         self._actor_descs = (ctypes.POINTER(_lib.NetDesc) * n)(*[ctypes.pointer(self.actors[a].layout.desc) for a in self.agent_ids])
-        self._critic_descs = (ctypes.POINTER(_lib.NetDesc) * n)(*[ctypes.pointer(self.critics[a].layout.desc) for a in self.agent_ids])
+        self._critic_descs = (ctypes.POINTER(_lib.NetDesc) * n)(*[ctypes.pointer(critics[a].layout.desc) for a in self.agent_ids])
         self._ws: dict = {}
-        self._all_opts = list(self.actor_optimizers.values()) + list(self.critic_optimizers.values())
+        self._all_opts = [o for name in self._opt_names() for o in getattr(self, name).values()]
         self._lib = _lib.load()
         self._drop_plans()
         if "use_graph" not in self.__dict__:
@@ -198,9 +219,15 @@ class MADDPG(EvolvableAlgorithm):
         except Exception:  # noqa: BLE001 - interpreter shutdown
             pass
 
+    def _opt_names(self) -> list:
+        return ["actor_optimizers"] + [opt for _, _, opt in self._CRITIC_SETS]
+
+    def _net_names(self) -> list:
+        """Every network set, each evaluation network followed by its target."""
+        return ["actors", "actor_targets"] + [x for net, tgt, _ in self._CRITIC_SETS for x in (net, tgt)]
+
     def _opt_state(self) -> dict:
-        return {"actors": {a: o.state_dict() for a, o in self.actor_optimizers.items()},
-                "critics": {a: o.state_dict() for a, o in self.critic_optimizers.items()}}
+        return {name: {a: o.state_dict() for a, o in getattr(self, name).items()} for name in self._opt_names()}
 
     def reinit_optimizers(self, optimizer=None) -> None:
         self._bind_engine()
@@ -211,9 +238,10 @@ class MADDPG(EvolvableAlgorithm):
             for o in self.__dict__.get("actor_optimizers", {}).values():
                 o.lr = value
         if name == "lr_critic":
-            for o in self.__dict__.get("critic_optimizers", {}).values():
-                o.lr = value
-        if name in ("lr_actor", "lr_critic", "gamma", "tau", "concurrent_agents") and self.__dict__.get("_plans"):
+            for _, _, opt in self._CRITIC_SETS:
+                for o in self.__dict__.get(opt, {}).values():
+                    o.lr = value
+        if name in ("lr_actor", "lr_critic", "gamma", "tau", "policy_freq", "concurrent_agents") and self.__dict__.get("_plans"):
             self._drop_plans()                     # these scalars are baked into a captured call
 
     def clone(self, index: int | None = None, wrap: bool = True):
@@ -223,16 +251,15 @@ class MADDPG(EvolvableAlgorithm):
         kw["device"] = self.device
         c = type(self)(**kw)
         for a in self.agent_ids:
-            for src, dst in ((self.actors, c.actors), (self.actor_targets, c.actor_targets), (self.critics, c.critics),
-                             (self.critic_targets, c.critic_targets)):
-                dst[a].buffers.copy_from(src[a].buffers)
+            for name in self._net_names():
+                getattr(c, name)[a].buffers.copy_from(getattr(self, name)[a].buffers)
         c._bind_engine(keep=self._opt_state())
         c.use_graph, c.concurrent_agents = self.use_graph, self.concurrent_agents
         c.expl_noise = {a: v.clone() for a, v in self.expl_noise.items()}
         c.mean_noise = {a: v.clone() for a, v in self.mean_noise.items()}
         c.current_noise = {a: v.clone() for a, v in self.current_noise.items()}
         c.scores, c.fitness, c.steps = list(self.scores), list(self.fitness), list(self.steps)
-        c.learn_counter = self.learn_counter
+        c.learn_counter = copy.deepcopy(self.learn_counter)
         return c
 
     # -- cross-rank move (population sharding: hpo/tournament.py::_select_sharded broadcasts a winner from its owner) ------
@@ -246,17 +273,26 @@ class MADDPG(EvolvableAlgorithm):
     def _state_tensors(self) -> list:
         out = []
         for a in self.agent_ids:
-            ao, co = self.actor_optimizers[a], self.critic_optimizers[a]
-            out += [self.actors[a].buffers.params, self.actor_targets[a].buffers.params, self.critics[a].buffers.params,
-                    self.critic_targets[a].buffers.params, ao.exp_avg, ao.exp_avg_sq, co.exp_avg, co.exp_avg_sq]
+            out += [getattr(self, name)[a].buffers.params for name in self._net_names()]
+            for name in self._opt_names():
+                o = getattr(self, name)[a]
+                out += [o.exp_avg, o.exp_avg_sq]
         return out
+
+    def _restore_steps(self, attrs: dict) -> None:
+        """Adam step counts from ``export_state``'s attributes: per optimiser set where recorded, else the one count."""
+        steps = attrs.get("opt_steps", {})
+        for name in self._opt_names():
+            for o in getattr(self, name).values():
+                o.step = steps.get(name, attrs["opt_step"])
 
     def export_state(self):
         """-> (picklable description, [device tensors]): every network's flat parameter buffer and both Adam moments of
-        every optimiser, 8 tensors per agent (≈ 0.5 MB for config 5)."""
+        every optimiser, 8 tensors per agent for MADDPG (≈ 0.5 MB for config 5), 12 for MATD3."""
         meta = {"init": self._init_kwargs(),
                 "attrs": {"scores": list(self.scores), "fitness": list(self.fitness), "steps": list(self.steps), "index": self.index,
-                          "learn_counter": self.learn_counter, "opt_step": self._all_opts[-1].step,
+                          "learn_counter": copy.deepcopy(self.learn_counter), "opt_step": self._all_opts[-1].step,
+                          "opt_steps": {name: next(iter(getattr(self, name).values())).step for name in self._opt_names()},
                           "expl_noise": self.expl_noise, "mean_noise": self.mean_noise, "current_noise": self.current_noise}}
         return meta, self._state_tensors()
 
@@ -267,9 +303,8 @@ class MADDPG(EvolvableAlgorithm):
             dst.copy_(src)
         a = meta["attrs"]
         agent.scores, agent.fitness, agent.steps, agent.index = a["scores"], a["fitness"], a["steps"], a["index"]
-        agent.learn_counter = a["learn_counter"]
-        for o in agent._all_opts:
-            o.step = a["opt_step"]
+        agent.learn_counter = copy.deepcopy(a["learn_counter"])
+        agent._restore_steps(a)
         agent.expl_noise, agent.mean_noise, agent.current_noise = a["expl_noise"], a["mean_noise"], a["current_noise"]
         return agent
 
@@ -289,17 +324,17 @@ class MADDPG(EvolvableAlgorithm):
         mine = self._state_tensors()
         if len(mine) != len(tensors) or any(tuple(a.shape) != tuple(b.shape) for a, b in zip(mine, tensors)):
             raise ValueError("checkpoint networks do not fit this member's architecture")
-        for k in ("batch_size", "lr_actor", "lr_critic", "learn_step", "gamma", "tau", "mut"):
-            setattr(self, k, init[k])
+        for k in ("batch_size", "lr_actor", "lr_critic", "learn_step", "gamma", "tau", "mut", "policy_freq"):
+            if k in init:
+                setattr(self, k, init[k])
         if init.get("hp_config") is not None:
             self.hp_config = self.registry.hp_config = init["hp_config"]
         for dst, src in zip(mine, tensors):
             dst.copy_(src)
         a = meta["attrs"]
         self.scores, self.fitness, self.steps, self.index = a["scores"], a["fitness"], a["steps"], a["index"]
-        self.learn_counter = a["learn_counter"]
-        for o in self._all_opts:
-            o.step = a["opt_step"]
+        self.learn_counter = copy.deepcopy(a["learn_counter"])
+        self._restore_steps(a)
         self.expl_noise, self.mean_noise, self.current_noise = a["expl_noise"], a["mean_noise"], a["current_noise"]
 
     @classmethod
@@ -417,9 +452,13 @@ class MADDPG(EvolvableAlgorithm):
         ws = self._ws.get(B)
         if ws is None:
             need = ctypes.c_size_t(0)
-            _lib.check(_lib.load().b2rl_maddpg_workspace_bytes(ctypes.cast(self._actor_descs, ctypes.c_void_p),
-                                                               ctypes.cast(self._critic_descs, ctypes.c_void_p), self.n_agents, B,
-                                                               ctypes.byref(need)))
+            actors, critics = ctypes.cast(self._actor_descs, ctypes.c_void_p), ctypes.cast(self._critic_descs, ctypes.c_void_p)
+            if len(self._CRITIC_SETS) == 2:            # a twin call also holds the critic_2 passes
+                cfg = _lib.MaddpgCfg()
+                cfg.batch, cfg.n_agents, cfg.twin = B, self.n_agents, 1
+                _lib.check(_lib.load().b2rl_maddpg_workspace_bytes_cfg(actors, critics, ctypes.byref(cfg), ctypes.byref(need)))
+            else:
+                _lib.check(_lib.load().b2rl_maddpg_workspace_bytes(actors, critics, self.n_agents, B, ctypes.byref(need)))
             ws = self._ws[B] = torch.empty(need.value, dtype=torch.uint8, device=self._dev)
         return ws
 
@@ -435,10 +474,30 @@ class MADDPG(EvolvableAlgorithm):
         return m
 
     def learn(self, experiences) -> dict:
-        """maddpg.py:571-628.  Returns ``{agent_id: (actor_loss, critic_loss)}`` as Python floats."""
+        """maddpg.py:571-628.  Returns ``{agent_id: (actor_loss, critic_loss)}`` as Python floats (MATD3: ``None`` for the
+        actor loss of a call without an actor step)."""
+        critic_only = self._next_critic_only()
         out = self.learn_device(experiences)
         host = out.tolist()
-        return {a: (host[i][0], host[i][1]) for i, a in enumerate(self.agent_ids)}
+        return {a: (None if critic_only else host[i][0], host[i][1]) for i, a in enumerate(self.agent_ids)}
+
+    # -- step kinds: MADDPG steps every optimiser and soft-updates every target on every call ------------------------
+    def _next_critic_only(self) -> bool:
+        """Whether the NEXT learn call updates the critics only (no actor step, no soft update)."""
+        return False
+
+    def _advance(self) -> bool:
+        """Count the learn call about to run: optimiser step counts and ``learn_counter``.  -> its step kind."""
+        for o in self._all_opts:
+            o.step += 1
+        self.learn_counter += 1
+        return False
+
+    def _bias_corrections(self, cfg) -> None:
+        a_step = max(next(iter(self.actor_optimizers.values())).step, 1)
+        c_step = max(next(iter(getattr(self, self._CRITIC_SETS[0][2]).values())).step, 1)
+        cfg.bc1_actor, cfg.bc2_actor = 1.0 - 0.9 ** a_step, 1.0 - 0.999 ** a_step
+        cfg.bc1_critic, cfg.bc2_critic = 1.0 - 0.9 ** c_step, 1.0 - 0.999 ** c_step
 
     def batch_buffers(self, B: int) -> list:
         """The static ``[B, sum]`` matrices a captured learn call reads, in the replay's field order (obs, action, reward,
@@ -452,35 +511,42 @@ class MADDPG(EvolvableAlgorithm):
             plan = self._plans[B] = _LearnPlan(self, B)
         return plan
 
-    def _call_args(self, B, obs, next_obs, act, rew, done, out, state_dev=None):
+    def _call_args(self, B, obs, next_obs, act, rew, done, out, state_dev=None, critic_only=False, actor_state_dev=None):
         n = self.n_agents
         cfg = _lib.MaddpgCfg()
         cfg.batch, cfg.n_agents, cfg.serial = B, n, int(not self.concurrent_agents)
         cfg.gamma, cfg.tau = float(self.gamma), float(self.tau)
         cfg.lr_actor, cfg.lr_critic, cfg.beta1, cfg.beta2, cfg.adam_eps = float(self.lr_actor), float(self.lr_critic), 0.9, 0.999, 1e-8
-        a_step = max(next(iter(self.actor_optimizers.values())).step, 1)
-        c_step = max(next(iter(self.critic_optimizers.values())).step, 1)
-        cfg.bc1_actor, cfg.bc2_actor = 1.0 - 0.9 ** a_step, 1.0 - 0.999 ** a_step
-        cfg.bc1_critic, cfg.bc2_critic = 1.0 - 0.9 ** c_step, 1.0 - 0.999 ** c_step
+        cfg.twin, cfg.critic_only = int(len(self._CRITIC_SETS) == 2), int(critic_only)
+        self._bias_corrections(cfg)
         bufs = _lib.MaddpgBufs()
         for i, a in enumerate(self.agent_ids):
-            ao, co = self.actor_optimizers[a], self.critic_optimizers[a]
+            ao = self.actor_optimizers[a]
             bufs.actor[i], bufs.actor_target[i] = self.actors[a].buffers.params.data_ptr(), self.actor_targets[a].buffers.params.data_ptr()
             bufs.actor_grads[i], bufs.actor_m[i], bufs.actor_v[i] = ao.grads.data_ptr(), ao.exp_avg.data_ptr(), ao.exp_avg_sq.data_ptr()
-            bufs.critic[i], bufs.critic_target[i] = self.critics[a].buffers.params.data_ptr(), self.critic_targets[a].buffers.params.data_ptr()
-            bufs.critic_grads[i], bufs.critic_m[i], bufs.critic_v[i] = co.grads.data_ptr(), co.exp_avg.data_ptr(), co.exp_avg_sq.data_ptr()
+            for k, (net, tgt, opt) in enumerate(self._CRITIC_SETS):
+                co = getattr(self, opt)[a]
+                pre = "critic" if k == 0 else "critic2"
+                getattr(bufs, pre)[i] = getattr(self, net)[a].buffers.params.data_ptr()
+                getattr(bufs, pre + "_target")[i] = getattr(self, tgt)[a].buffers.params.data_ptr()
+                getattr(bufs, pre + "_grads")[i], getattr(bufs, pre + "_m")[i] = co.grads.data_ptr(), co.exp_avg.data_ptr()
+                getattr(bufs, pre + "_v")[i] = co.exp_avg_sq.data_ptr()
         bufs.obs, bufs.next_obs, bufs.action = obs.data_ptr(), next_obs.data_ptr(), act.data_ptr()
         bufs.reward, bufs.done = rew.data_ptr(), done.data_ptr()
         bufs.losses = out.data_ptr()
         ws = self._workspace(B)
         bufs.workspace, bufs.workspace_bytes = ws.data_ptr(), ws.numel()
         bufs.step_state = state_dev.data_ptr() if state_dev is not None else None
+        bufs.actor_step_state = actor_state_dev.data_ptr() if actor_state_dev is not None else None
         return cfg, bufs
 
-    def _capture(self, plan: _LearnPlan, B: int) -> None:
+    def _capture(self, plan: _LearnPlan, B: int, critic_only: bool = False) -> None:
         lib = _lib.load()
-        cfg, bufs = self._call_args(B, plan.obs, plan.next_obs, plan.action, plan.reward, plan.done, plan.out, plan.state_dev)
-        plan._keep = (cfg, bufs)
+        # separate actor bias corrections: only a twin (MATD3) full step, whose actors lag the critics
+        actor_state = plan.actor_state_dev if (len(self._CRITIC_SETS) == 2 and not critic_only) else None
+        cfg, bufs = self._call_args(B, plan.obs, plan.next_obs, plan.action, plan.reward, plan.done, plan.out, plan.state_dev,
+                                    critic_only, actor_state)
+        plan.__dict__.setdefault("_keep", {})[critic_only] = (cfg, bufs)
         cap = torch.cuda.Stream(device=self._dev)
         cap.wait_stream(torch.cuda.current_stream(self._dev))
         s = cap.cuda_stream
@@ -488,31 +554,34 @@ class MADDPG(EvolvableAlgorithm):
         _lib.check(lib.b2rl_graph_begin(s))
         try:
             _lib.check(lib.b2rl_step_state_write(ctypes.byref(plan.state_host), plan.state_dev.data_ptr(), s))
+            if actor_state is not None:
+                _lib.check(lib.b2rl_step_state_write(ctypes.byref(plan.actor_state_host), actor_state.data_ptr(), s))
             _lib.check(lib.b2rl_maddpg_learn(ctypes.cast(self._actor_descs, ctypes.c_void_p),
                                              ctypes.cast(self._critic_descs, ctypes.c_void_p), ctypes.byref(cfg), ctypes.byref(bufs), s))
         finally:
             _lib.check(lib.b2rl_graph_end(s, ctypes.byref(gh)))
-        plan.graph = gh.value
+        plan.graphs[critic_only] = gh.value
         torch.cuda.current_stream(self._dev).wait_stream(cap)
 
     def graph_ready(self, B: int) -> bool:
-        """A captured learn call for batch size ``B`` exists (the next ``learn_device`` on ``batch_buffers(B)`` is one
-        graph launch and touches no torch state: it may be given an explicit stream)."""
+        """A captured learn call for batch size ``B`` and the next call's step kind exists (the next ``learn_device`` on
+        ``batch_buffers(B)`` is one graph launch and touches no torch state: it may be given an explicit stream)."""
         plan = self._plans.get(B)
-        return bool(self.use_graph and plan is not None and plan.graph is not None)
+        return bool(self.use_graph and plan is not None and plan.graphs.get(self._next_critic_only()) is not None)
 
     def learn_device(self, experiences, stream: int | None = None) -> torch.Tensor:
-        """``learn`` without the host read-back: device tensor ``[n_agents, 2]`` (actor_loss, critic_loss).  With
-        ``use_graph`` the tensor is the plan's static result buffer: valid until the next learn call of this batch size.
-        ``stream`` (raw ``cudaStream_t``; only when ``graph_ready`` and the batch sits in ``batch_buffers``): launch there
-        instead of on torch's current stream."""
+        """``learn`` without the host read-back: device tensor ``[n_agents, 2]`` (actor_loss, critic_loss; the actor column
+        is NaN after a MATD3 call without an actor step).  With ``use_graph`` the tensor is the plan's static result buffer:
+        valid until the next learn call of this batch size.  ``stream`` (raw ``cudaStream_t``; only when ``graph_ready``
+        and the batch sits in ``batch_buffers``): launch there instead of on torch's current stream."""
         states, actions, rewards, next_states, dones = experiences
+        critic_only = self._next_critic_only()
         if self.use_graph:          # the replay gathered straight into a captured call's buffers: nothing to check or copy
             p = getattr(states, "packed", None)
             plan = self._plans.get(p.shape[0]) if p is not None else None
-            if (plan is not None and plan.graph is not None and p is plan.obs and getattr(actions, "packed", None) is plan.action
-                    and getattr(rewards, "packed", None) is plan.reward and getattr(next_states, "packed", None) is plan.next_obs
-                    and getattr(dones, "packed", None) is plan.done):
+            if (plan is not None and plan.graphs.get(critic_only) is not None and p is plan.obs
+                    and getattr(actions, "packed", None) is plan.action and getattr(rewards, "packed", None) is plan.reward
+                    and getattr(next_states, "packed", None) is plan.next_obs and getattr(dones, "packed", None) is plan.done):
                 return self._replay(plan, stream)
         assert stream is None, "an explicit stream is only valid for a captured call on batch_buffers()"
         n = self.n_agents
@@ -527,15 +596,13 @@ class MADDPG(EvolvableAlgorithm):
             for dst, src in zip(plan.fields(), (obs, act, rew, next_obs, done)):
                 if dst.data_ptr() != src.data_ptr():
                     dst.copy_(src)
-            if plan.graph is None:
+            if plan.graphs.get(critic_only) is None:
                 self._workspace(B)                                # also creates the library's side streams: not under capture
-                self._capture(plan, B)
+                self._capture(plan, B, critic_only)
             return self._replay(plan)
-        for o in self._all_opts:
-            o.step += 1
-        self.learn_counter += 1
+        critic_only = self._advance()
         out = torch.empty((n, 2), dtype=torch.float32, device=self._dev)
-        cfg, bufs = self._call_args(B, obs, next_obs, act, rew, done, out)
+        cfg, bufs = self._call_args(B, obs, next_obs, act, rew, done, out, critic_only=critic_only)
         _lib.check(lib.b2rl_maddpg_learn(ctypes.cast(self._actor_descs, ctypes.c_void_p),
                                          ctypes.cast(self._critic_descs, ctypes.c_void_p), ctypes.byref(cfg), ctypes.byref(bufs),
                                          _lib.stream_ptr(self._dev)))
@@ -543,13 +610,15 @@ class MADDPG(EvolvableAlgorithm):
         return out
 
     def _replay(self, plan: _LearnPlan, stream: int | None = None) -> torch.Tensor:
-        for o in self._all_opts:
-            o.step += 1
-        self.learn_counter += 1
+        critic_only = self._advance()
+        self._launch(plan, plan.graphs[critic_only], critic_only, _lib.stream_ptr(self._dev) if stream is None else stream)
+        return plan.out
+
+    def _launch(self, plan: _LearnPlan, graph, critic_only: bool, stream: int) -> None:
+        """Replay a captured call with this step's Adam bias corrections (MADDPG: every optimiser's step count is one)."""
         step = self._all_opts[-1].step
         plan.state_host.bias_correction1, plan.state_host.bias_correction2 = 1.0 - 0.9 ** step, 1.0 - 0.999 ** step
-        _lib.check(self._lib.b2rl_graph_launch(plan.graph, plan.state_ref, _lib.stream_ptr(self._dev) if stream is None else stream))
-        return plan.out
+        _lib.check(self._lib.b2rl_graph_launch(graph, plan.state_ref, stream))
 
     def soft_update(self, net, target) -> None:
         """maddpg.py:733-746."""

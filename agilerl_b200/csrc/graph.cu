@@ -22,6 +22,10 @@ struct b2rl_graph {
     cudaGraphNode_t state_node = nullptr;
     cudaKernelNodeParams state_params{};
     b2rl_step_state *state_dev = nullptr;
+    // every step_state_write_kernel node with its destination (the first of them is state_node above)
+    std::vector<cudaGraphNode_t> state_nodes;
+    std::vector<cudaKernelNodeParams> state_node_params;
+    std::vector<b2rl_step_state *> state_dsts;
     int kernels = 0;
 };
 
@@ -64,10 +68,15 @@ int b2rl_graph_end(void *stream, b2rl_graph **out_host) {
         ++g->kernels;
         cudaKernelNodeParams p{};
         B2RL_CUDA(cudaGraphKernelNodeGetParams(nodes[i], &p));
-        if (p.func == (void *)step_state_write_kernel && g->state_node == nullptr) {
+        if (p.func != (void *)step_state_write_kernel) continue;
+        b2rl_step_state *dst = *reinterpret_cast<b2rl_step_state **>(p.kernelParams[1]);
+        g->state_nodes.push_back(nodes[i]);
+        g->state_node_params.push_back(p);
+        g->state_dsts.push_back(dst);
+        if (g->state_node == nullptr) {
             g->state_node = nodes[i];
             g->state_params = p;
-            g->state_dev = *reinterpret_cast<b2rl_step_state **>(p.kernelParams[1]);
+            g->state_dev = dst;
         }
     }
     B2RL_CUDA(cudaGraphInstantiate(&g->exec, graph, 0));
@@ -86,6 +95,28 @@ int b2rl_graph_launch(b2rl_graph *g, const b2rl_step_state *state_host, void *st
         p.kernelParams = args;
         p.extra = nullptr;
         B2RL_CUDA(cudaGraphExecKernelNodeSetParams(g->exec, g->state_node, &p));
+    }
+    B2RL_CUDA(cudaGraphLaunch(g->exec, as_stream(stream)));
+    g_launches += (unsigned long long)g->kernels;
+    return B2RL_OK;
+}
+
+int b2rl_graph_launch_states(b2rl_graph *g, const b2rl_step_state *const *states_host, b2rl_step_state *const *states_dev, int n,
+                             void *stream) {
+    B2RL_CHECK_ARG(g && g->exec, "NULL graph");
+    B2RL_CHECK_ARG(n >= 0 && (n == 0 || (states_host && states_dev)), "bad step-state arguments");
+    for (int k = 0; k < n; ++k) {
+        B2RL_CHECK_ARG(states_host[k] != nullptr, "NULL host step state %d", k);
+        size_t j = 0;
+        while (j < g->state_dsts.size() && g->state_dsts[j] != states_dev[k]) ++j;
+        B2RL_CHECK_ARG(j < g->state_dsts.size(), "no step-state write node of this graph writes state %d", k);
+        b2rl_step_state v = *states_host[k];
+        b2rl_step_state *dst = g->state_dsts[j];
+        void *args[2] = {&v, &dst};
+        cudaKernelNodeParams p = g->state_node_params[j];
+        p.kernelParams = args;
+        p.extra = nullptr;
+        B2RL_CUDA(cudaGraphExecKernelNodeSetParams(g->exec, g->state_nodes[j], &p));
     }
     B2RL_CUDA(cudaGraphLaunch(g->exec, as_stream(stream)));
     g_launches += (unsigned long long)g->kernels;

@@ -54,6 +54,38 @@ __global__ void maddpg_td_loss_kernel(const float *__restrict__ q, const float *
     if (threadIdx.x == 0) *loss = s / (float)B;
 }
 
+// matd3.py:769-788, the twin-critic TD step: y = r + (1 - d) * gamma * min(Q'1, Q'2) with maddpg_td_loss_kernel's
+// NaN handling; critic_loss = MSE(Q1, y) + MSE(Q2, y); seeds dL/dQk = 2 (Qk - y) / B.  One CTA, fixed-order sums.
+// actor_loss != NULL (a critic-only call, no actor step): NaN there, so a device-side reader never sees a stale value.
+__global__ void matd3_td_loss_kernel(const float *__restrict__ q1, const float *__restrict__ q2, const float *__restrict__ qn1,
+                                     const float *__restrict__ qn2, const float *__restrict__ reward, const float *__restrict__ done,
+                                     int ld, float gamma, int64_t B, float *__restrict__ g1, float *__restrict__ g2,
+                                     float *__restrict__ loss, float *__restrict__ actor_loss) {
+    __shared__ float red[32];
+    float s1 = 0.f, s2 = 0.f;
+    for (int64_t i = threadIdx.x; i < B; i += blockDim.x) {
+        float r = reward[i * ld], d = done[i * ld];
+        r = isnan(r) ? 0.f : r;
+        d = isnan(d) ? 1.f : d;
+        const unsigned d8 = __float2uint_rz(fminf(fmaxf(d, 0.f), 255.f)) & 0xFFu;      // .to(torch.uint8)
+        const float omd = (float)((1u - d8) & 0xFFu);
+        const float a = qn1[i], b = qn2[i];
+        const float qn = (isnan(a) || a < b) ? a : b;                                   // torch.min: NaN propagates
+        const float y = __fadd_rn(r, __fmul_rn(__fmul_rn(omd, gamma), qn));
+        const float d1 = q1[i] - y, d2 = q2[i] - y;
+        s1 += d1 * d1;
+        s2 += d2 * d2;
+        g1[i] = 2.0f * d1 / (float)B;
+        g2[i] = 2.0f * d2 / (float)B;
+    }
+    s1 = block_reduce_sum(s1, red);
+    s2 = block_reduce_sum(s2, red);
+    if (threadIdx.x == 0) {
+        *loss = s1 / (float)B + s2 / (float)B;
+        if (actor_loss) *actor_loss = __int_as_float(0x7fc00000);
+    }
+}
+
 // hpo/mutation.py:733-827 on the device: slot j mutates W[rows[j]][cols[j]] (host-drawn positions and branch
 // uniforms, the reference's numpy stream).  branch: u < 0.05 -> w + |10 w| z; u < 0.10 -> z; else w + |sd w| z;
 // clamp(+-1e6).  keep[j] == 0 marks a slot whose position is written again by a later slot (index_put_: last writer
@@ -76,8 +108,8 @@ __global__ void gaussian_mutate_kernel(float *__restrict__ W, int64_t ld, const 
     }
 }
 
-// torch.optim.Adam (no clipping) + the Polyak update of the target, one flat parameter buffer.  state != NULL (a
-// captured learn call): this step's bias corrections come from the device block the graph's first node rewrites —
+// torch.optim.Adam (no clipping) + the Polyak update of the target, one flat parameter buffer (tgt == NULL: Adam only, a
+// MATD3 call without soft updates).  state != NULL (a captured learn call): this step's bias corrections come from the device block the graph's first node rewrites —
 // the same double arithmetic as the host's (lr / bc1, sqrt(bc2)), so a replay is bit-identical to the eager call.
 __global__ void ma_adam_polyak_kernel(float *__restrict__ p, const float *__restrict__ g, float *__restrict__ m,
                                       float *__restrict__ v, float *__restrict__ tgt, int64_t n, AdamCfg c, double lr,
@@ -95,7 +127,7 @@ __global__ void ma_adam_polyak_kernel(float *__restrict__ p, const float *__rest
         const float denom = sqrtf(vi) / c.bc2_sqrt + c.eps;
         const float pi = p[i] + (c.neg_step * mi) / denom;   // addcdiv_(exp_avg, denom, value=-step_size)
         p[i] = pi;
-        tgt[i] = __fadd_rn(__fmul_rn(c.tau, pi), __fmul_rn(c.one_minus_tau, tgt[i]));   // soft_update (maddpg.py:733-746)
+        if (tgt) tgt[i] = __fadd_rn(__fmul_rn(c.tau, pi), __fmul_rn(c.one_minus_tau, tgt[i]));   // soft_update (maddpg.py:733-746)
     }
 }
 static int ma_adam(float *p, float *g, float *m, float *v, float *tgt, int64_t n, double lr, double bc1, double bc2,
@@ -116,9 +148,14 @@ static int ma_adam(float *p, float *g, float *m, float *v, float *tgt, int64_t n
 // steps are independent of each other — own networks, own optimiser state, own scratch — so they run concurrently
 // and the call's critical path is one agent's chain instead of n.  Library-owned, created once per process; forked
 // from and joined back into the caller's stream with events, which a stream capture turns into graph edges.
+// A twin call (MATD3) gives every agent a second stream, s[B2RL_MAX_AGENTS + i], for its critic_2 chains: forwards,
+// backward and Adam of critic_2 depend on critic_1's only through the TD step, and the actor step reads critic_1 alone.
 struct MaStreams {
-    cudaStream_t s[B2RL_MAX_AGENTS] = {};
+    cudaStream_t s[2 * B2RL_MAX_AGENTS] = {};
     cudaEvent_t fork = nullptr, ta[B2RL_MAX_AGENTS] = {}, join[B2RL_MAX_AGENTS] = {};
+    // twin: fork2 (agent stream -> critic_2 stream), q2 (critic_2's Q values are ready for the TD step), td (its
+    // gradient seed is written), join2 (critic_2 stepped)
+    cudaEvent_t fork2[B2RL_MAX_AGENTS] = {}, q2[B2RL_MAX_AGENTS] = {}, td[B2RL_MAX_AGENTS] = {}, join2[B2RL_MAX_AGENTS] = {};
     bool ready = false;
 };
 static int ma_streams(MaStreams **out) {
@@ -127,8 +164,9 @@ static int ma_streams(MaStreams **out) {
         B2RL_CUDA(cudaEventCreateWithFlags(&ms.fork, cudaEventDisableTiming));
         for (int i = 0; i < B2RL_MAX_AGENTS; ++i) {
             B2RL_CUDA(cudaStreamCreateWithFlags(&ms.s[i], cudaStreamNonBlocking));
-            B2RL_CUDA(cudaEventCreateWithFlags(&ms.ta[i], cudaEventDisableTiming));
-            B2RL_CUDA(cudaEventCreateWithFlags(&ms.join[i], cudaEventDisableTiming));
+            B2RL_CUDA(cudaStreamCreateWithFlags(&ms.s[B2RL_MAX_AGENTS + i], cudaStreamNonBlocking));
+            for (cudaEvent_t *e : {&ms.ta[i], &ms.join[i], &ms.fork2[i], &ms.q2[i], &ms.td[i], &ms.join2[i]})
+                B2RL_CUDA(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
         }
         ms.ready = true;
     }
@@ -146,6 +184,10 @@ struct MaAgentWS {
     float *act_mod;                  // [B, sum act] the batch's actions with agent i's columns replaced
     float *g_obs;                    // dL/d(input) scratch of the first chains (unused result)
     float *lnpart;                   // LayerNorm-affine partial sums of this agent's backward passes
+    // twin only (carved after everything above, so a MADDPG workspace is unchanged): critic_2 passes [0] critic_2(obs, act)
+    // with gradients, [1] critic_2_target(next_obs, next_act); own dL/d(input) and LayerNorm scratch (its own stream)
+    LayerBuf c2_enc[2][B2RL_MAX_ENC], c2_head[2][B2RL_MAX_HEAD];
+    float *cat2[2], *g_cat2, *g_obs2, *lnpart2;
 };
 struct MaWS {
     MaAgentWS ag[B2RL_MAX_AGENTS];
@@ -183,7 +225,7 @@ static int ma_shape(const b2rl_net_desc *const *actors, const b2rl_net_desc *con
 }
 
 static void carve_maddpg(const b2rl_net_desc *const *actors, const b2rl_net_desc *const *critics, const MaShape &sh, int64_t B,
-                         void *base, MaWS &ws) {
+                         bool twin, void *base, MaWS &ws) {
     Bump b(base);
     const int SO = sh.o_off[sh.n], SA = sh.a_off[sh.n];
     ws.next_act = b.take<float>(B * SA);
@@ -209,6 +251,18 @@ static void carve_maddpg(const b2rl_net_desc *const *actors, const b2rl_net_desc
         w.obs_i = b.take<float>(B * a.enc[0].in_c);
         w.nobs_i = b.take<float>(B * a.enc[0].in_c);
     }
+    for (int i = 0; twin && i < sh.n; ++i) {     // critic_2 shares critic_1's description (same architecture)
+        MaAgentWS &w = ws.ag[i];
+        const b2rl_net_desc &c = *critics[i];
+        for (int p = 0; p < 2; ++p) {
+            carve_layers(b, c.enc, c.n_enc, w.c2_enc[p], B, p == 0 ? B : 0);
+            carve_layers(b, c.val, c.n_val, w.c2_head[p], B, p == 0 ? B : 0);
+            w.cat2[p] = b.take<float>(B * (sh.L + SA));
+        }
+        w.g_cat2 = b.take<float>(B * (sh.L + SA));
+        w.g_obs2 = b.take<float>(B * SO);
+        w.lnpart2 = b.take<float>(ws.lnpart_floats);
+    }
     ws.bytes = b.off + 256;
 }
 
@@ -228,18 +282,29 @@ using namespace b2rl;
 
 extern "C" {
 
-int b2rl_maddpg_workspace_bytes(const b2rl_net_desc *const *actors_host, const b2rl_net_desc *const *critics_host, int n_agents,
-                                int64_t batch, size_t *out_host) {
+static int maddpg_workspace_bytes(const b2rl_net_desc *const *actors_host, const b2rl_net_desc *const *critics_host, int n_agents,
+                                  int64_t batch, bool twin, size_t *out_host) {
     B2RL_CHECK_ARG(out_host && batch >= 1, "bad arguments");
     MaShape sh;
     int rc = ma_shape(actors_host, critics_host, n_agents, sh);
     if (rc != B2RL_OK) return rc;
     MaWS ws;
-    carve_maddpg(actors_host, critics_host, sh, batch, nullptr, ws);
+    carve_maddpg(actors_host, critics_host, sh, batch, twin, nullptr, ws);
     *out_host = ws.bytes;
     MaStreams *ms;                       // everything a later stream capture must not create: side streams, events,
     if ((rc = ma_streams(&ms)) != B2RL_OK) return rc;     // kernel attributes
     return head_kernels_ready();
+}
+
+int b2rl_maddpg_workspace_bytes(const b2rl_net_desc *const *actors_host, const b2rl_net_desc *const *critics_host, int n_agents,
+                                int64_t batch, size_t *out_host) {
+    return maddpg_workspace_bytes(actors_host, critics_host, n_agents, batch, false, out_host);
+}
+
+int b2rl_maddpg_workspace_bytes_cfg(const b2rl_net_desc *const *actors_host, const b2rl_net_desc *const *critics_host,
+                                    const b2rl_maddpg_cfg *cfg_host, size_t *out_host) {
+    B2RL_CHECK_ARG(cfg_host, "NULL descriptor");
+    return maddpg_workspace_bytes(actors_host, critics_host, cfg_host->n_agents, cfg_host->batch, cfg_host->twin != 0, out_host);
 }
 
 int b2rl_maddpg_learn(const b2rl_net_desc *const *actors_host, const b2rl_net_desc *const *critics_host,
@@ -249,27 +314,33 @@ int b2rl_maddpg_learn(const b2rl_net_desc *const *actors_host, const b2rl_net_de
     const b2rl_maddpg_bufs &bf = *bufs_host;
     const int64_t B = cfg.batch;
     const int n = cfg.n_agents;
+    const bool twin = cfg.twin != 0, critic_only = cfg.critic_only != 0;
     B2RL_CHECK_ARG(B >= 1, "Batch size must be greater than or equal to one.");
     MaShape sh;
     int rc = ma_shape(actors_host, critics_host, n, sh);
     if (rc != B2RL_OK) return rc;
     B2RL_CHECK_ARG(bf.obs && bf.next_obs && bf.action && bf.reward && bf.done && bf.losses, "NULL batch buffer");
-    for (int i = 0; i < n; ++i)
+    for (int i = 0; i < n; ++i) {
         B2RL_CHECK_ARG(bf.actor[i] && bf.actor_target[i] && bf.actor_grads[i] && bf.actor_m[i] && bf.actor_v[i] && bf.critic[i] &&
                            bf.critic_target[i] && bf.critic_grads[i] && bf.critic_m[i] && bf.critic_v[i],
                        "NULL network buffer of agent %d", i);
+        B2RL_CHECK_ARG(!twin || (bf.critic2[i] && bf.critic2_target[i] && bf.critic2_grads[i] && bf.critic2_m[i] && bf.critic2_v[i]),
+                       "NULL critic_2 buffer of agent %d", i);
+    }
     MaWS ws;
-    carve_maddpg(actors_host, critics_host, sh, B, bf.workspace, ws);
+    carve_maddpg(actors_host, critics_host, sh, B, twin, bf.workspace, ws);
     B2RL_CHECK_ARG(bf.workspace && bf.workspace_bytes >= ws.bytes, "workspace too small: need %zu bytes, got %zu", ws.bytes,
                    bf.workspace_bytes);
     cudaStream_t s = as_stream(stream);
     const int SO = sh.o_off[n], SA = sh.a_off[n], L = sh.L;
     const b2rl_step_state *state = static_cast<const b2rl_step_state *>(bf.step_state);
+    const b2rl_step_state *actor_state = bf.actor_step_state ? static_cast<const b2rl_step_state *>(bf.actor_step_state) : state;
     const bool fan = !cfg.serial && n > 1;
+    const bool fan2 = !cfg.serial && twin;
     MaStreams *ms = nullptr;
-    if (fan) {
+    if (fan || fan2) {
         if ((rc = ma_streams(&ms)) != B2RL_OK) return rc;
-        B2RL_CUDA(cudaEventRecord(ms->fork, s));
+        if (fan) B2RL_CUDA(cudaEventRecord(ms->fork, s));
     }
 
     // (0) next actions of every agent from the target actors (maddpg.py:600-609), side by side like torch.cat(dim=1)
@@ -296,15 +367,56 @@ int b2rl_maddpg_learn(const b2rl_net_desc *const *actors_host, const b2rl_net_de
                 if (j != i) B2RL_CUDA(cudaStreamWaitEvent(si, ms->ta[j], 0));
         const Chain ae = enc_chain(a), ah = val_chain(a), ce = enc_chain(c), ch = val_chain(c);
         const int o = sh.o_off[i + 1] - sh.o_off[i], ad = sh.a_off[i + 1] - sh.a_off[i];
-        // (1) Q_i(obs, act) and the target Q'_i(next_obs, next_act)
+        cudaStream_t s2 = fan2 ? ms->s[B2RL_MAX_AGENTS + i] : si;
+        if (fan2) {
+            B2RL_CUDA(cudaEventRecord(ms->fork2[i], si));
+            B2RL_CUDA(cudaStreamWaitEvent(s2, ms->fork2[i], 0));
+        }
+        // (1) Q_i(obs, act) and the target Q'_i(next_obs, next_act) (twin: the same two passes of critic_2 on s2)
+        if (twin) {
+            if ((rc = ma_critic_forward(c, bf.critic2[i], bf.obs, bf.action, B, w.c2_enc[0], w.c2_head[0], w.cat2[0], L, SA, s2)) != B2RL_OK)
+                return rc;
+            if ((rc = ma_critic_forward(c, bf.critic2_target[i], bf.next_obs, ws.next_act, B, w.c2_enc[1], w.c2_head[1], w.cat2[1], L, SA,
+                                        s2)) != B2RL_OK)
+                return rc;
+            if (fan2) B2RL_CUDA(cudaEventRecord(ms->q2[i], s2));
+        }
         if ((rc = ma_critic_forward(c, bf.critic[i], bf.obs, bf.action, B, w.c_enc[0], w.c_head[0], w.cat[0], L, SA, si)) != B2RL_OK) return rc;
         if ((rc = ma_critic_forward(c, bf.critic_target[i], bf.next_obs, ws.next_act, B, w.c_enc[1], w.c_head[1], w.cat[1], L, SA, si)) != B2RL_OK)
             return rc;
         // (2) TD target, MSE, dL/dq seed
-        maddpg_td_loss_kernel<<<1, 512, 0, si>>>(w.c_head[0][c.n_val - 1].a, w.c_head[1][c.n_val - 1].a, bf.reward + i, bf.done + i, n,
-                                                 (float)cfg.gamma, B, w.c_head[0][c.n_val - 1].g, bf.losses + 2 * i + 1);
-        B2RL_LAUNCH_CHECK();
-        // (3) critic backward + Adam + Polyak
+        if (twin) {
+            if (fan2) B2RL_CUDA(cudaStreamWaitEvent(si, ms->q2[i], 0));
+            matd3_td_loss_kernel<<<1, 512, 0, si>>>(w.c_head[0][c.n_val - 1].a, w.c2_head[0][c.n_val - 1].a, w.c_head[1][c.n_val - 1].a,
+                                                    w.c2_head[1][c.n_val - 1].a, bf.reward + i, bf.done + i, n, (float)cfg.gamma, B,
+                                                    w.c_head[0][c.n_val - 1].g, w.c2_head[0][c.n_val - 1].g, bf.losses + 2 * i + 1,
+                                                    critic_only ? bf.losses + 2 * i : nullptr);
+            B2RL_LAUNCH_CHECK();
+            if (fan2) {
+                B2RL_CUDA(cudaEventRecord(ms->td[i], si));
+                B2RL_CUDA(cudaStreamWaitEvent(s2, ms->td[i], 0));
+            }
+        } else {
+            maddpg_td_loss_kernel<<<1, 512, 0, si>>>(w.c_head[0][c.n_val - 1].a, w.c_head[1][c.n_val - 1].a, bf.reward + i, bf.done + i, n,
+                                                     (float)cfg.gamma, B, w.c_head[0][c.n_val - 1].g, bf.losses + 2 * i + 1);
+            B2RL_LAUNCH_CHECK();
+            if (critic_only) B2RL_CUDA(cudaMemsetAsync(bf.losses + 2 * i, 0xFF, sizeof(float), si));     // all-ones bits: a NaN
+        }
+        // (3) critic backward + Adam (+ Polyak unless critic-only); twin: critic_2's on s2, beside critic_1's
+        if (twin) {
+            if ((rc = chain_backward(ch, bf.critic2[i], w.cat2[0], B, w.c2_head[0], w.g_cat2, bf.critic2_grads[i], w.lnpart2,
+                                     ws.lnpart_floats, s2)) != B2RL_OK)
+                return rc;
+            ddpg_slice_kernel<<<ew_blocks(B * L), 256, 0, s2>>>(w.g_cat2, L + SA, 0, L, B, w.c2_enc[0][c.n_enc - 1].g);
+            B2RL_LAUNCH_CHECK();
+            if ((rc = chain_backward(ce, bf.critic2[i], bf.obs, B, w.c2_enc[0], w.g_obs2, bf.critic2_grads[i], w.lnpart2, ws.lnpart_floats,
+                                     s2)) != B2RL_OK)
+                return rc;
+            if ((rc = ma_adam(bf.critic2[i], bf.critic2_grads[i], bf.critic2_m[i], bf.critic2_v[i], critic_only ? nullptr : bf.critic2_target[i],
+                              c.n_params, cfg.lr_critic, cfg.bc1_critic, cfg.bc2_critic, cfg, state, s2)) != B2RL_OK)
+                return rc;
+            if (fan2) B2RL_CUDA(cudaEventRecord(ms->join2[i], s2));
+        }
         if ((rc = chain_backward(ch, bf.critic[i], w.cat[0], B, w.c_head[0], w.g_cat[0], bf.critic_grads[i], w.lnpart,
                                  ws.lnpart_floats, si)) != B2RL_OK)
             return rc;
@@ -313,33 +425,38 @@ int b2rl_maddpg_learn(const b2rl_net_desc *const *actors_host, const b2rl_net_de
         if ((rc = chain_backward(ce, bf.critic[i], bf.obs, B, w.c_enc[0], w.g_obs, bf.critic_grads[i], w.lnpart, ws.lnpart_floats,
                                  si)) != B2RL_OK)
             return rc;
-        if ((rc = ma_adam(bf.critic[i], bf.critic_grads[i], bf.critic_m[i], bf.critic_v[i], bf.critic_target[i], c.n_params,
-                          cfg.lr_critic, cfg.bc1_critic, cfg.bc2_critic, cfg, state, si)) != B2RL_OK)
+        if ((rc = ma_adam(bf.critic[i], bf.critic_grads[i], bf.critic_m[i], bf.critic_v[i], critic_only ? nullptr : bf.critic_target[i],
+                          c.n_params, cfg.lr_critic, cfg.bc1_critic, cfg.bc2_critic, cfg, state, si)) != B2RL_OK)
             return rc;
         // (4) actor step through the UPDATED critic_i: -mean Q_i(obs, [act_0 .. actor_i(obs_i) .. act_n-1])
-        ddpg_slice_kernel<<<ew_blocks(B * o), 256, 0, si>>>(bf.obs, SO, sh.o_off[i], o, B, w.obs_i);
-        B2RL_LAUNCH_CHECK();
-        if ((rc = chain_forward(ae, bf.actor[i], w.obs_i, B, w.a_enc[0], si)) != B2RL_OK) return rc;
-        if ((rc = chain_forward(ah, bf.actor[i], w.a_enc[0][a.n_enc - 1].a, B, w.a_head[0], si)) != B2RL_OK) return rc;
-        B2RL_CUDA(cudaMemcpyAsync(w.act_mod, bf.action, sizeof(float) * B * SA, cudaMemcpyDeviceToDevice, si));
-        maddpg_put_cols_kernel<<<ew_blocks(B * ad), 256, 0, si>>>(w.a_head[0][a.n_val - 1].a, ad, w.act_mod, SA, sh.a_off[i], B);
-        B2RL_LAUNCH_CHECK();
-        if ((rc = ma_critic_forward(c, bf.critic[i], bf.obs, w.act_mod, B, w.c_enc[2], w.c_head[2], w.cat[2], L, SA, si)) != B2RL_OK) return rc;
-        ddpg_actor_loss_kernel<<<1, 512, 0, si>>>(w.c_head[2][c.n_val - 1].a, B, w.c_head[2][c.n_val - 1].g, bf.losses + 2 * i);
-        B2RL_LAUNCH_CHECK();
-        if ((rc = chain_backward(ch, bf.critic[i], w.cat[2], B, w.c_head[2], w.g_cat[2], nullptr, w.lnpart, ws.lnpart_floats, si)) != B2RL_OK)
-            return rc;
-        ddpg_slice_kernel<<<ew_blocks(B * ad), 256, 0, si>>>(w.g_cat[2], L + SA, L + sh.a_off[i], ad, B, w.a_head[0][a.n_val - 1].g);
-        B2RL_LAUNCH_CHECK();
-        if ((rc = chain_backward(ah, bf.actor[i], w.a_enc[0][a.n_enc - 1].a, B, w.a_head[0], w.a_enc[0][a.n_enc - 1].g,
-                                 bf.actor_grads[i], w.lnpart, ws.lnpart_floats, si)) != B2RL_OK)
-            return rc;
-        if ((rc = chain_backward(ae, bf.actor[i], w.obs_i, B, w.a_enc[0], w.g_obs, bf.actor_grads[i], w.lnpart, ws.lnpart_floats,
-                                 si)) != B2RL_OK)
-            return rc;
-        if ((rc = ma_adam(bf.actor[i], bf.actor_grads[i], bf.actor_m[i], bf.actor_v[i], bf.actor_target[i], a.n_params,
-                          cfg.lr_actor, cfg.bc1_actor, cfg.bc2_actor, cfg, state, si)) != B2RL_OK)
-            return rc;
+        if (!critic_only) {
+            ddpg_slice_kernel<<<ew_blocks(B * o), 256, 0, si>>>(bf.obs, SO, sh.o_off[i], o, B, w.obs_i);
+            B2RL_LAUNCH_CHECK();
+            if ((rc = chain_forward(ae, bf.actor[i], w.obs_i, B, w.a_enc[0], si)) != B2RL_OK) return rc;
+            if ((rc = chain_forward(ah, bf.actor[i], w.a_enc[0][a.n_enc - 1].a, B, w.a_head[0], si)) != B2RL_OK) return rc;
+            B2RL_CUDA(cudaMemcpyAsync(w.act_mod, bf.action, sizeof(float) * B * SA, cudaMemcpyDeviceToDevice, si));
+            maddpg_put_cols_kernel<<<ew_blocks(B * ad), 256, 0, si>>>(w.a_head[0][a.n_val - 1].a, ad, w.act_mod, SA, sh.a_off[i], B);
+            B2RL_LAUNCH_CHECK();
+            if ((rc = ma_critic_forward(c, bf.critic[i], bf.obs, w.act_mod, B, w.c_enc[2], w.c_head[2], w.cat[2], L, SA, si)) != B2RL_OK)
+                return rc;
+            ddpg_actor_loss_kernel<<<1, 512, 0, si>>>(w.c_head[2][c.n_val - 1].a, B, w.c_head[2][c.n_val - 1].g, bf.losses + 2 * i);
+            B2RL_LAUNCH_CHECK();
+            if ((rc = chain_backward(ch, bf.critic[i], w.cat[2], B, w.c_head[2], w.g_cat[2], nullptr, w.lnpart, ws.lnpart_floats, si)) !=
+                B2RL_OK)
+                return rc;
+            ddpg_slice_kernel<<<ew_blocks(B * ad), 256, 0, si>>>(w.g_cat[2], L + SA, L + sh.a_off[i], ad, B, w.a_head[0][a.n_val - 1].g);
+            B2RL_LAUNCH_CHECK();
+            if ((rc = chain_backward(ah, bf.actor[i], w.a_enc[0][a.n_enc - 1].a, B, w.a_head[0], w.a_enc[0][a.n_enc - 1].g,
+                                     bf.actor_grads[i], w.lnpart, ws.lnpart_floats, si)) != B2RL_OK)
+                return rc;
+            if ((rc = chain_backward(ae, bf.actor[i], w.obs_i, B, w.a_enc[0], w.g_obs, bf.actor_grads[i], w.lnpart, ws.lnpart_floats,
+                                     si)) != B2RL_OK)
+                return rc;
+            if ((rc = ma_adam(bf.actor[i], bf.actor_grads[i], bf.actor_m[i], bf.actor_v[i], bf.actor_target[i], a.n_params,
+                              cfg.lr_actor, cfg.bc1_actor, cfg.bc2_actor, cfg, actor_state, si)) != B2RL_OK)
+                return rc;
+        }
+        if (fan2) B2RL_CUDA(cudaStreamWaitEvent(si, ms->join2[i], 0));
         if (fan) B2RL_CUDA(cudaEventRecord(ms->join[i], si));
     }
     if (fan)

@@ -130,7 +130,7 @@ class Mutations:
         policy = getattr(individual, registry.policy())
         if isinstance(policy, dict):
             raise NotImplementedError("architecture mutations of multi-agent networks (mutation.py:887-1010) are not implemented "
-                                      "on the CUDA path: use parameter / RL hyper-parameter mutations for MADDPG")
+                                      "on the CUDA path: use parameter / RL hyper-parameter mutations for MADDPG / MATD3")
         if not policy.mutation_methods:
             individual.mut = "None"
             return individual

@@ -55,7 +55,7 @@ _MEMBER_STREAMS: dict = {}
 
 
 def multi_agent_population_learn(pop, memory, batch_size: int | None = None, overlap: bool = True) -> list:
-    """One learn call of every member of a MADDPG population (all on one device) against the shared HBM replay
+    """One learn call of every member of a MADDPG or MATD3 population (all on one device) against the shared HBM replay
     (train_multi_agent_off_policy: ``experiences = memory.sample(agent.batch_size); agent.learn(experiences)`` per
     member).  The members share nothing that a learn call writes — the replay is only read — so each member's position
     draw, gather (straight into the buffers its captured learn call reads) and graph launch go to the member's own

@@ -1,6 +1,6 @@
 """``train_multi_agent_off_policy`` — same signature and control flow as
-agilerl/training/train_multi_agent_off_policy.py:32-600 for the multi-agent learner of this package (MADDPG), minus the
-W&B / accelerate plumbing and image-observation channel swapping (the CUDA MADDPG takes vector observations).  The reference's
+agilerl/training/train_multi_agent_off_policy.py:32-600 for the multi-agent learners of this package (MADDPG, MATD3), minus the
+W&B / accelerate plumbing and image-observation channel swapping (the CUDA learners take vector observations).  The reference's
 file cannot be imported on the GPU box (pettingzoo / accelerate / wandb are absent there), so this module restates its loop;
 ``tests/test_reference_driver_cpu.py`` runs both files on the same seeded population, environment and stand-in kernels and
 requires identical fitnesses, scores, steps, mutations and replay contents.
@@ -41,7 +41,7 @@ def train_multi_agent_off_policy(env, env_name: str, algo: str, pop: list, memor
     if wb or accelerator is not None:
         raise NotImplementedError("W&B logging / accelerate are outside this package (the population shards one process per GPU)")
     if swap_channels:
-        raise NotImplementedError("image observations are not implemented for MADDPG on the CUDA path")
+        raise NotImplementedError(f"image observations are not implemented for {algo} on the CUDA path")
     if save_elite is False and elite_path is not None:
         warnings.warn("'save_elite' set to False but 'elite_path' has been defined, elite will not be saved unless 'save_elite' "
                       "is set to True.", stacklevel=2)

@@ -1,11 +1,11 @@
 """Population helpers — mirrors of agilerl/utils/utils.py:218-653 (``create_population`` for the
-learners of this package: DQN, Rainbow DQN, DDPG, TD3, MADDPG) and :706-796 (``tournament_selection_and_mutation``, the
+learners of this package: DQN, Rainbow DQN, DDPG, TD3, MADDPG, MATD3) and :706-796 (``tournament_selection_and_mutation``, the
 non-accelerate branch :785-786)."""
 from __future__ import annotations
 
 from typing import Any
 
-from ..algorithms import DDPG, DQN, MADDPG, TD3, RainbowDQN
+from ..algorithms import DDPG, DQN, MADDPG, MATD3, TD3, RainbowDQN
 
 
 def create_population(algo: str, observation_space, action_space, net_config: dict | None, INIT_HP: dict,
@@ -15,8 +15,8 @@ def create_population(algo: str, observation_space, action_space, net_config: di
     """utils/utils.py:218-474.  ``first_index`` numbers the agents of a population shard."""
     population = []
     algo_kwargs = algo_kwargs or {}
-    if algo == "MADDPG" and INIT_HP.get("SHARE_ENCODERS", False):
-        raise NotImplementedError("SHARE_ENCODERS is not implemented for MADDPG on the CUDA path")
+    if algo in ("MADDPG", "MATD3") and INIT_HP.get("SHARE_ENCODERS", False):
+        raise NotImplementedError(f"SHARE_ENCODERS is not implemented for {algo} on the CUDA path")
     noise = dict(O_U_noise=INIT_HP.get("O_U_NOISE", True), expl_noise=INIT_HP.get("EXPL_NOISE", 0.1), vect_noise_dim=num_envs,
                  mean_noise=INIT_HP.get("MEAN_NOISE", 0.0), theta=INIT_HP.get("THETA", 0.15), dt=INIT_HP.get("DT", 0.01))
     pg = dict(hp_config=hp_config, net_config=net_config, batch_size=INIT_HP.get("BATCH_SIZE", 64),
@@ -55,8 +55,14 @@ def create_population(algo: str, observation_space, action_space, net_config: di
                            index=idx, gamma=INIT_HP.get("GAMMA", 0.95), tau=INIT_HP.get("TAU", 0.01),
                            actor_networks=actor_network, critic_networks=critic_network, torch_compiler=torch_compiler,
                            **noise, **pg, **algo_kwargs)
+        elif algo == "MATD3":                                                   # utils.py:474-500
+            agent = MATD3(observation_spaces=observation_space, action_spaces=action_space, agent_ids=INIT_HP["AGENT_IDS"],
+                          index=idx, policy_freq=INIT_HP.get("POLICY_FREQ", 2), gamma=INIT_HP.get("GAMMA", 0.95),
+                          tau=INIT_HP.get("TAU", 0.01), actor_networks=actor_network, critic_networks=critic_network,
+                          torch_compiler=torch_compiler, **noise, **pg, **algo_kwargs)
         else:
-            raise NotImplementedError(f"{algo}: not one of the learners of this package (DQN, Rainbow DQN, DDPG, TD3, MADDPG; SURVEY §8)")
+            raise NotImplementedError(f"{algo}: not one of the learners of this package (DQN, Rainbow DQN, DDPG, TD3, MADDPG, MATD3; "
+                                      "SURVEY §8)")
         population.append(agent)
     return population
 

@@ -449,6 +449,13 @@ typedef struct b2rl_maddpg_cfg {
     double gamma, tau;
     double lr_actor, lr_critic, beta1, beta2, adam_eps;
     double bc1_actor, bc2_actor, bc1_critic, bc2_critic;   /* 1 - beta^step of the actor / critic optimisers */
+    /* MATD3 (agilerl/algorithms/matd3.py:630-831).  Both zero: the MADDPG call above. */
+    int32_t twin;                       /* 1: a second critic set (bufs.critic2*): y = r + (1 - d) gamma min(Q'1, Q'2),
+                                           critic_loss = MSE(Q1, y) + MSE(Q2, y), both critics step; the actor step
+                                           reads critic_1 only.  No target-policy smoothing noise (unlike TD3). */
+    int32_t critic_only;                /* 1: critic TD steps only — no actor forward / backward / Adam and no Polyak
+                                           update of any target (a MATD3 call where learn_counter % policy_freq != 0);
+                                           losses[i][0] is written NaN */
 } b2rl_maddpg_cfg;
 
 typedef struct b2rl_maddpg_bufs {
@@ -463,12 +470,22 @@ typedef struct b2rl_maddpg_bufs {
     void *workspace; size_t workspace_bytes;
     const b2rl_step_state *step_state;  /* nullable (device): a captured call reads this step's Adam bias corrections
                                            (bias_correction1 / 2; every optimiser steps once per call) from here */
+    /* twin only: critic_2 of every agent, its target, gradients and Adam moments (critic_1's architecture) */
+    float *critic2[B2RL_MAX_AGENTS], *critic2_target[B2RL_MAX_AGENTS], *critic2_grads[B2RL_MAX_AGENTS],
+          *critic2_m[B2RL_MAX_AGENTS], *critic2_v[B2RL_MAX_AGENTS];
+    const b2rl_step_state *actor_step_state;   /* nullable (device): the ACTOR optimisers' bias corrections of a captured
+                                                  call whose actors and critics have stepped different numbers of times
+                                                  (MATD3); NULL: the actors read step_state too */
 } b2rl_maddpg_bufs;
 
 int b2rl_maddpg_workspace_bytes(const b2rl_net_desc *const *actors_host, const b2rl_net_desc *const *critics_host, int n_agents,
                                 int64_t batch, size_t *out_host);
+/* The same for the call cfg_host describes (batch, n_agents, twin): a twin call needs room for the critic_2 passes. */
+int b2rl_maddpg_workspace_bytes_cfg(const b2rl_net_desc *const *actors_host, const b2rl_net_desc *const *critics_host,
+                                    const b2rl_maddpg_cfg *cfg_host, size_t *out_host);
 /* One learn call of every agent, then every soft update (fused into the optimiser launches: no target is read after its
- * network stepped).  actors_host / critics_host: n_agents pointers to the (host) layer tables. */
+ * network stepped).  actors_host / critics_host: n_agents pointers to the (host) layer tables (critic_2 of a twin call
+ * shares critic_1's table).  Side streams (serial == 0): one per agent, plus one per agent for critic_2's chains. */
 int b2rl_maddpg_learn(const b2rl_net_desc *const *actors_host, const b2rl_net_desc *const *critics_host,
                       const b2rl_maddpg_cfg *cfg_host, const b2rl_maddpg_bufs *bufs_host, void *stream);
 
@@ -498,6 +515,11 @@ int b2rl_graph_begin(void *stream);
 int b2rl_graph_end(void *stream, b2rl_graph **out_host);
 /* state_host may be NULL when the graph holds no b2rl_step_state_write node. */
 int b2rl_graph_launch(b2rl_graph *g, const b2rl_step_state *state_host, void *stream);
+/* For a graph with several b2rl_step_state_write nodes (e.g. a MATD3 policy call: critic and actor bias corrections):
+ * the node that writes states_dev[k] gets *states_host[k], k < n; every state_dev given must have a node in the graph,
+ * nodes not named keep their last value. */
+int b2rl_graph_launch_states(b2rl_graph *g, const b2rl_step_state *const *states_host, b2rl_step_state *const *states_dev, int n,
+                             void *stream);
 /* kernel nodes in the graph (what one replay adds to b2rl_launch_count) */
 int b2rl_graph_kernel_count(const b2rl_graph *g, int *out_host);
 int b2rl_graph_destroy(b2rl_graph *g);
